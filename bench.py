@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline metric of the exact-scan hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (mmr_search: scan + top-k) over the whole index for one batch of B
 queries.  Workload = BASELINE.json's metric config: exact top-10 over a synthetic 10M x 512 bf16 CLIP-shaped
@@ -70,7 +70,14 @@ def parse():
     ap.add_argument("--exchange", default="auto", choices=["auto", "fused", "nccl"],
                     help="N>1: fused = peer-memory stores from the scan kernel + wait/merge kernel; nccl = all-gather + merge")
     ap.add_argument("--sweep", default="8,128,1024", help="extra batch sizes reported under 'sweep' (N=1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy, so two "
+                    "builds can be compared output for output (same arguments = same inputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the B200 path's results (the CPU arm may scan a sample of the rows)")
+    return args
 
 
 def measured_peaks():
@@ -103,11 +110,32 @@ def load_traffic():
 
 
 # --------------------------------------------------------------------------------------------- synthetic data
-def gen_block_f32(block_id: int, rows: int, dim: int, device):
-    import torch
-    g = torch.Generator(device=device)
-    g.manual_seed(SEED * 1_000_003 + block_id)
-    return torch.randn((rows, dim), generator=g, device=device, dtype=torch.float32)
+def host_block(block_id: int, n: int, dim: int, out=None) -> np.ndarray:
+    """The first n rows of block `block_id` of the synthetic table: normalised N(0,1)^dim in fp32, seeded by
+    (SEED, block id).  The generator fills rows in order, so a shorter block is a prefix of a longer one."""
+    blk = np.empty((n, dim), dtype=np.float32) if out is None else out
+    rng = np.random.default_rng([SEED, block_id])
+    rng.standard_normal(out=blk, dtype=np.float32)
+    blk /= np.sqrt(np.einsum("ij,ij->i", blk, blk))[:, None]
+    return blk
+
+
+def table_blocks(lo: int, hi: int, dim: int, threads: int):
+    """Rows [lo, hi) of the synthetic table as (first row, fp32 rows) pairs, equal to host_table(n)[lo:hi] for every
+    n >= hi.  Blocks are generated `threads` at a time, so at most that many are held in host memory."""
+    from concurrent.futures import ThreadPoolExecutor
+
+    threads = max(1, threads)
+    b0, b1 = lo // BLOCK_ROWS, (hi + BLOCK_ROWS - 1) // BLOCK_ROWS
+
+    def make(b):
+        s = b * BLOCK_ROWS
+        cs, ce = max(s, lo), min(s + BLOCK_ROWS, hi)
+        return cs, host_block(b, ce - s, dim)[cs - s:]
+
+    with ThreadPoolExecutor(threads) as pool:
+        for c in range(b0, b1, threads):
+            yield from pool.map(make, range(c, min(c + threads, b1)))
 
 
 def gen_queries(n: int, dim: int):
@@ -118,23 +146,13 @@ def gen_queries(n: int, dim: int):
 
 
 def build_shard(pkg, lo: int, hi: int, dim: int, dtype: str, device):
-    """Rows [lo, hi) of the synthetic table, generated on the device block by block, normalised + narrowed by
-    the loader kernel (mmr_convert_rows_f32, normalize=1)."""
+    """Rows [lo, hi) of the synthetic table, the same rows host_table generates, narrowed on the device by the L1
+    loader B200Store.load_arrow uses (mmr_load_rows_f32_host_scatter): one table whichever way a run loads it."""
     import torch
-    N = pkg._native
     tdt = {"bf16": torch.bfloat16, "f16": torch.float16, "f32": torch.float32}[dtype]
-    code = {"bf16": N.MMR_BF16, "f16": N.MMR_F16, "f32": N.MMR_F32}[dtype]
     rows = torch.empty((hi - lo, dim), dtype=tdt, device=device)
-    stream = torch.cuda.current_stream(device).cuda_stream
-    b0, b1 = lo // BLOCK_ROWS, (hi + BLOCK_ROWS - 1) // BLOCK_ROWS
-    for b in range(b0, b1):
-        s, e = b * BLOCK_ROWS, (b + 1) * BLOCK_ROWS
-        blk = gen_block_f32(b, BLOCK_ROWS, dim, device)
-        cs, ce = max(s, lo), min(e, hi)
-        src = blk[cs - s:ce - s]
-        N.check(N.lib().mmr_convert_rows_f32(src.data_ptr(), rows[cs - lo:ce - lo].data_ptr(), code, ce - cs, dim, 1, stream))
-        torch.cuda.synchronize(device)
-        del blk, src
+    for start, blk in table_blocks(lo, hi, dim, min(host_cores(), 8)):
+        pkg.ResidentIndex.load_rows_into(rows, blk, dst_offset=start - lo)
     return pkg.ResidentIndex(rows, row_base=lo)
 
 
@@ -152,6 +170,22 @@ def planted_rows(n_rows: int, bounds, world: int, k: int):
         if len(planted) == k:
             break
     return sorted(planted)
+
+
+def dump_outputs(dirname: str, arrays: dict, limit: int = 64 << 20) -> None:
+    """Write each [B, ...] result array as dirname/<name>.npy: floats as float32, integers (row ids) as float64, both
+    exact.  Above `limit` bytes in all, every array keeps the same seeded sample of its B queries, whose indices go to
+    query_index.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    out = {name: a.astype(np.float32 if a.dtype.kind == "f" else np.float64) for name, a in arrays.items()}
+    n = len(next(iter(out.values())))
+    per_query = sum(a.nbytes for a in out.values()) // max(n, 1) + 8
+    if per_query * n > limit:
+        keep = np.sort(np.random.default_rng(SEED).choice(n, limit // per_query, replace=False))
+        out = {name: a[keep] for name, a in out.items()}
+        out["query_index"] = keep.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 # --------------------------------------------------------------------------------------------- clocks
@@ -233,10 +267,7 @@ def host_table(n: int, dim: int, threads: int) -> np.ndarray:
 
     def fill(b):
         s, e = b * BLOCK_ROWS, min((b + 1) * BLOCK_ROWS, n)
-        rng = np.random.default_rng([SEED, b])
-        blk = out[s:e]
-        rng.standard_normal(out=blk, dtype=np.float32)
-        blk /= np.sqrt(np.einsum("ij,ij->i", blk, blk))[:, None]
+        host_block(b, e - s, dim, out=out[s:e])
 
     with ThreadPoolExecutor(max(1, threads)) as pool:
         list(pool.map(fill, range((n + BLOCK_ROWS - 1) // BLOCK_ROWS)))
@@ -312,11 +343,10 @@ def run_reference(args):
     n_warm = max(1, min(args.warmup, 3))
     for i in range(n_warm):
         cpu.search(qs[i % len(qs)], args.k)
-    steps = 0
+    steps = args.steps
     t0 = time.perf_counter()
-    while steps < max(1, args.steps) and (steps < 3 or time.perf_counter() - t0 < 120.0):
-        cpu.search(qs[args.warmup + steps], args.k)
-        steps += 1
+    for i in range(steps):
+        cpu.search(qs[args.warmup + i], args.k)
     dt = (time.perf_counter() - t0) / steps * cpu.scale
     qps = args.batch / dt
     desc = cpu.describe()
@@ -365,6 +395,7 @@ def run_b200(args):
     esize = 4 if args.dtype == "f32" else 2
     q_host = gen_queries((K + W) * B, D).reshape(K + W, B, D)
     planted = planted_rows(args.rows, bounds, world, k)
+    unit_q0 = q_host[0, 0] / np.linalg.norm(q_host[0, 0])
 
     # N = 1: the table goes the way a deployment loads it -- fp32 rows in the reference's Arrow schema ->
     # B200Store.load_arrow (columnar host copy, scatter loader fp32 -> resident bf16) -- and every number below is taken
@@ -377,7 +408,6 @@ def run_b200(args):
         use_store = cpu.scale == 1.0            # the whole table fits host memory
     if use_store:
         import pyarrow as pa
-        unit_q0 = q_host[0, 0] / np.linalg.norm(q_host[0, 0])
         cpu.table[planted] = unit_q0              # the parity rows are part of the table itself (host AND device copy)
         n = args.rows
         t0 = time.perf_counter()
@@ -410,10 +440,10 @@ def run_b200(args):
     # ---- parity inside the bench run: k exact copies of warm-up query 0 are planted on both sides of every shard
     # boundary (and at the table's first / last row); the search must return exactly those rows, in row order, with
     # equal scores, and -- for N > 1 -- the fused peer-memory exchange must equal the NCCL all-gather path bit for bit.
-    if not use_store:
+    if not use_store:   # through the store's loader, so both ways of loading hold the same planted rows
         mine = [c for c in planted if lo <= c < hi]
         if mine:
-            ix.rows[torch.tensor([c - lo for c in mine], device=device)] = q_dev[0, 0].to(ix.rows.dtype)
+            pkg.ResidentIndex.load_rows_into(ix.rows, np.tile(unit_q0, (len(mine), 1)), dst_rows=np.array(mine) - lo)
     torch.cuda.synchronize(device)
     pq = q_dev[0, :1].contiguous()
     if world > 1:
@@ -457,6 +487,8 @@ def run_b200(args):
     ms_step = ms_total / K
     qps = B / (ms_step * 1e-3)
     last_scores, last_rows = res[0].cpu().numpy(), res[1].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"scores": last_scores, "rows": last_rows})
 
     # kernel-only pass (no collective) for the roofline of the dominant kernel: one launch per step
     ev2, ev3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
