@@ -261,7 +261,10 @@ int mmr_encoder_create(int device, const mmr_encoder_config* config, mmr_encoder
 int mmr_encoder_destroy(mmr_encoder* encoder);
 int mmr_encoder_out_dim(const mmr_encoder* encoder);
 int mmr_encoder_set_weight(mmr_encoder* encoder, const char* name, const float* data_dev, int64_t numel, void* stream);
-/* One forward pass for B sequences padded to S tokens (S <= 512).  ids / mask (1 = token, 0 = padding; NULL = all ones) /
+/* One forward pass for B sequences padded to S tokens.  S <= 512, except S <= 330 for a model with head dim 64 whose
+ * attention runs on the fp32 kernel: the query encoders (MMR_ENC_MINILM, MMR_ENC_CLIP_TEXT) unless MMR_ENC_ATT_MMA=2 (the
+ * cross-encoder's tensor-core attention takes 512 at either head dim).  Longer sequences fail with MMR_ERR_UNSUPPORTED.
+ * ids / mask (1 = token, 0 = padding; NULL = all ones) /
  * token types (NULL = all zero) are HOST arrays [B, S]; out_dev is [B, out_dim] fp32 on the encoder's device
  * (L2-normalised embeddings, or [B] logits for MMR_ENC_CROSS) -- directly usable as mmr_search's queries_dev. */
 int mmr_encoder_forward(mmr_encoder* encoder, const int32_t* input_ids_host, const int32_t* attention_mask_host,
@@ -275,6 +278,33 @@ int mmr_encoder_forward(mmr_encoder* encoder, const int32_t* input_ids_host, con
 int mmr_debug_umma_scores(const mmr_index* index, const float* queries_dev, int32_t B, int64_t row_begin,
                           int64_t row_end, float* out_scores_dev, int64_t out_ld, void* workspace_dev,
                           size_t workspace_bytes, void* stream);
+
+/*
+ * Validation hooks for the encoder kernels: each runs ONE launch of the kernel the forward pass runs, through the same
+ * launch code, on caller-owned device buffers (row-major).  Arguments are checked before any CUDA call (MMR_ERR_INVALID
+ * with a message).
+ *   mmr_debug_enc_gemm       gemm_wt_kernel: out[t, f] = epilogue(sum_k X[t, k] W[f, k] + bias[f]), t < M, f < N.
+ *       epi       0 out_f32 = y; 1 out_f32 = y + residual (residual may equal out_f32: the in-place residual stream);
+ *                 2 out_bf16 = GELU(erf)(y); 3 out_bf16 = quick-GELU(y)
+ *       nt        token tile 64, 128 or 256 (box rows of X's tensor map)
+ *       fold_ln   0: x_dev is X bf16 [M, K].  1: X = bf16(LayerNorm(ln_src_dev fp32 [M, K]; ln_g, ln_b, ln_eps)) computed
+ *                 inside the GEMM (nt 64, K 384 or 512, epi != 1), the normalised rows also written to ln_out_dev fp32 [M, K]
+ *                 when it is not NULL (must not alias ln_src)
+ *       W bf16 [N, K]; N a multiple of 128, K of 64; bias fp32 [N] or NULL; residual / out_f32 fp32 [M, N]; out_bf16 bf16 [M, N]
+ *   mmr_debug_enc_attention  softmax(q k^T / sqrt(H / heads)) v per (sequence, head) over qkv fp32 [B * S, 3H] (q | k | v)
+ *       -> ctx bf16 [B * S, H]; tensor_cores 1 = attention_mma_kernel, 0 = attention_kernel; mask int32 [B * S] (0 = padding
+ *       key) or NULL; causal hides keys after the query row.  Sequence limits as for mmr_encoder_forward.
+ *   mmr_debug_enc_layernorm  layernorm_kernel<H>, H 384 or 512: rows of x fp32 [M, H] -> out_f32 (may equal x) and / or
+ *       out_bf16 bf16 [M, H].
+ */
+int mmr_debug_enc_gemm(int32_t epi, int32_t nt, int32_t fold_ln, int32_t M, int32_t N, int32_t K, const void* x_dev,
+                       const float* ln_src_dev, const float* ln_g_dev, const float* ln_b_dev, float ln_eps, float* ln_out_dev,
+                       const void* w_dev, const float* bias_dev, const float* residual_dev, float* out_f32_dev,
+                       void* out_bf16_dev, void* stream);
+int mmr_debug_enc_attention(int32_t tensor_cores, int32_t B, int32_t S, int32_t H, int32_t heads, int32_t causal,
+                            const float* qkv_dev, const int32_t* mask_dev, void* ctx_dev, void* stream);
+int mmr_debug_enc_layernorm(int32_t H, int32_t M, const float* x_dev, const float* g_dev, const float* b_dev, float eps,
+                            float* out_f32_dev, void* out_bf16_dev, void* stream);
 
 /* Introspection used by bench.py / tests: launches issued by this library since load, device facts. */
 int64_t mmr_launch_count(void);

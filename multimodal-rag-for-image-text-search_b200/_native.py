@@ -51,6 +51,9 @@ SYMBOLS = [
     ("mmr_fuse", C.c_int, [_p, _p, _i32, _p, _p, _i32, _i32, _i32, _f64, _p, _p, _p, _p, _p, _p]),
     ("mmr_fuse_f64", C.c_int, [_p, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _f64, _p, _p, _p, _p]),
     ("mmr_debug_umma_scores", C.c_int, [_p, _p, _i32, _i64, _i64, _p, _i64, _p, _sz, _p]),
+    ("mmr_debug_enc_gemm", C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, C.c_float, _p, _p, _p, _p, _p, _p, _p]),
+    ("mmr_debug_enc_attention", C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p]),
+    ("mmr_debug_enc_layernorm", C.c_int, [_i32, _i32, _p, _p, _p, C.c_float, _p, _p, _p]),
     ("mmr_launch_count", _i64, []),
     ("mmr_device_sm_count", C.c_int, [C.c_int, C.POINTER(C.c_int)]),
     ("mmr_last_kernel", C.c_int, []),

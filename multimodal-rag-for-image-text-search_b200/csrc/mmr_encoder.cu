@@ -306,6 +306,53 @@ static int launch_gemm_ln(const CUtensorMap& mw, const CUtensorMap& any_x_map, i
   return MMR_OK;
 }
 
+// Shared memory of one attention launch, checked against the kernel's own limit (the opt-in size set below): the fp32
+// kernel holds K and V of the head in fp32 (head dim 64: 330 tokens at most), the tensor-core kernel in bf16 (512 fit).
+static int attention_smem(bool tensor_cores, int DH, int S, size_t* smem) {
+  if (tensor_cores) {
+    *smem = DH == 32 ? attention_mma_smem_bytes<32>(S) : attention_mma_smem_bytes<64>(S);
+    if (*smem > 200 * 1024)
+      return fail(MMR_ERR_UNSUPPORTED, "sequence length %d does not fit the tensor-core attention kernel (head dim %d)", S, DH);
+  } else {
+    *smem = DH == 32 ? attention_smem_bytes<32>(S) : attention_smem_bytes<64>(S);
+    if (*smem > 220 * 1024)
+      return fail(MMR_ERR_UNSUPPORTED, "sequence length %d does not fit the fp32 attention kernel (head dim %d: %d tokens at most)", S,
+                  DH, DH == 32 ? 552 : 330);
+  }
+  return MMR_OK;
+}
+
+// One attention launch over qkv fp32 [B * S, 3H] -> ctx bf16 [B * S, H]: attention_mma_kernel (tensor_cores) or
+// attention_kernel, head dim H / heads.  The forward pass and mmr_debug_enc_attention both launch through here.
+static int launch_attention(bool tensor_cores, int B, int S, int H, int heads, int causal, const float* qkv, const int32_t* mask,
+                            __nv_bfloat16* ctx, cudaStream_t st) {
+  const int DH = H / heads;
+  size_t smem = 0;
+  const int rc = attention_smem(tensor_cores, DH, S, &smem);
+  if (rc != MMR_OK) return rc;
+  static bool att_attr[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (!att_attr[dev & 63]) {
+    CUDA_TRY(cudaFuncSetAttribute(attention_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CUDA_TRY(cudaFuncSetAttribute(attention_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    CUDA_TRY(cudaFuncSetAttribute(attention_mma_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CUDA_TRY(cudaFuncSetAttribute(attention_mma_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    att_attr[dev & 63] = true;
+  }
+  const dim3 att_mma_grid(heads, B, (S + ATC_ROWS - 1) / ATC_ROWS);
+  if (tensor_cores && DH == 32)
+    CUDA_TRY(launch_pdl(attention_mma_kernel<32>, att_mma_grid, dim3(ATC_NW * 32), smem, st, qkv, mask, ctx, S, H, causal));
+  else if (tensor_cores)
+    CUDA_TRY(launch_pdl(attention_mma_kernel<64>, att_mma_grid, dim3(ATC_NW * 32), smem, st, qkv, mask, ctx, S, H, causal));
+  else if (DH == 32)
+    CUDA_TRY(launch_pdl(attention_kernel<32>, dim3(heads, B), dim3(ATT_NW * 32), smem, st, qkv, mask, ctx, S, H, causal));
+  else
+    CUDA_TRY(launch_pdl(attention_kernel<64>, dim3(heads, B), dim3(ATT_NW * 32), smem, st, qkv, mask, ctx, S, H, causal));
+  mmr_g_launches++;
+  return MMR_OK;
+}
+
 template <int H>
 static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t st) {
   const mmr_encoder_config& c = e->cfg;
@@ -325,25 +372,13 @@ static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t 
     e->maps_tokens = M;
     e->maps_narrow = options().enc_narrow_tiles;
   }
-  static bool att_attr[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!att_attr[dev & 63]) {
-    CUDA_TRY(cudaFuncSetAttribute(attention_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    CUDA_TRY(cudaFuncSetAttribute(attention_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    CUDA_TRY(cudaFuncSetAttribute(attention_mma_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    CUDA_TRY(cudaFuncSetAttribute(attention_mma_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    att_attr[dev & 63] = true;
-  }
   // the cross-encoder (rerank passages: 128-512 tokens) runs both attention contractions on the tensor cores, whatever the
   // sequence length (kernel choice by model, never by batch shape); MMR_ENC_ATT_MMA=0: fp32 kernel everywhere, =2: every model
   // from ATC_MIN_S tokens on (measurement)
   const int att_opt = options().enc_att_mma;
   const bool att_mma = att_opt == 2 ? S >= ATC_MIN_S : (att_opt == 1 && c.kind == MMR_ENC_CROSS);
-  const size_t att_mma_smem = DH == 32 ? attention_mma_smem_bytes<32>(S) : attention_mma_smem_bytes<64>(S);
-  const dim3 att_mma_grid(c.heads, B, (S + ATC_ROWS - 1) / ATC_ROWS);
-  const size_t att_smem = DH == 32 ? attention_smem_bytes<32>(S) : attention_smem_bytes<64>(S);
-  if (att_smem > 220 * 1024) return fail(MMR_ERR_UNSUPPORTED, "sequence length %d does not fit the attention kernel", S);
+  size_t att_smem = 0;
+  if (const int rc = attention_smem(att_mma, DH, S, &att_smem); rc != MMR_OK) return rc;   // before the first launch
 
   // embeddings
   if (clip)
@@ -380,19 +415,8 @@ static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t 
       rc = launch_gemm<EPI_BIAS_F32>(L.m_qkv, e->m_x16, e->nt_x, M, 3 * H, H, L.qkv_b, nullptr, e->qkv, nullptr, st);
     }
     if (rc != MMR_OK) return rc;
-    if (att_mma && DH == 32)
-      CUDA_TRY(launch_pdl(attention_mma_kernel<32>, att_mma_grid, dim3(ATC_NW * 32), att_mma_smem, st, e->qkv, e->d_mask, e->ctx16, S,
-                          H, clip ? 1 : 0));
-    else if (att_mma)
-      CUDA_TRY(launch_pdl(attention_mma_kernel<64>, att_mma_grid, dim3(ATC_NW * 32), att_mma_smem, st, e->qkv, e->d_mask, e->ctx16, S,
-                          H, clip ? 1 : 0));
-    else if (DH == 32)
-      CUDA_TRY(launch_pdl(attention_kernel<32>, dim3(c.heads, B), dim3(ATT_NW * 32), att_smem, st, e->qkv, e->d_mask, e->ctx16, S, H,
-                          clip ? 1 : 0));
-    else
-      CUDA_TRY(launch_pdl(attention_kernel<64>, dim3(c.heads, B), dim3(ATT_NW * 32), att_smem, st, e->qkv, e->d_mask, e->ctx16, S, H,
-                          clip ? 1 : 0));
-    mmr_g_launches++;
+    rc = launch_attention(att_mma, B, S, H, c.heads, clip ? 1 : 0, e->qkv, e->d_mask, e->ctx16, st);
+    if (rc != MMR_OK) return rc;
     if (clip) {
       // x = x + out_proj(ctx); h = LN2(x); x = x + fc2(quick_gelu(fc1(h)))
       rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_o, e->m_ctx16, e->nt_ctx, M, H, H, L.o_b, e->x, e->x, nullptr, st);
@@ -474,4 +498,95 @@ extern "C" int mmr_encoder_forward(mmr_encoder* e, const int32_t* input_ids_host
   CUDA_TRY(cudaMemcpyAsync(e->d_ids, e->h_stage, cap * 3 * 4, cudaMemcpyHostToDevice, st));
   if (e->cfg.hidden == 384) return forward_t<384>(e, B, S, out_dev, st);
   return forward_t<512>(e, B, S, out_dev, st);
+}
+
+// ------------------------------------------------------------------------------------------------ validation hooks
+// One launch of an encoder kernel on caller buffers, through the same launch code as the forward pass (tests compare each
+// with a float64 reference).  Arguments are checked before any CUDA call.
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+template <int EPI>
+static int debug_gemm_epi(int nt, bool fold_ln, int M, int N, int K, const void* x_dev, const float* ln_src_dev, const float* ln_g_dev,
+                          const float* ln_b_dev, float ln_eps, float* ln_out_dev, const void* w_dev, const float* bias_dev,
+                          const float* residual_dev, float* out_f32_dev, void* out_bf16_dev, cudaStream_t st) {
+  CUtensorMap mw, mx;
+  if (!make_map(&mw, w_dev, N, K, ENC_BM) || (!fold_ln && !make_map(&mx, x_dev, M, K, nt)))
+    return fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+  __nv_bfloat16* o16 = static_cast<__nv_bfloat16*>(out_bf16_dev);
+  if (fold_ln)   // the folded kernel never reads the activation map
+    return launch_gemm_ln<EPI>(mw, mw, M, N, K, bias_dev, out_f32_dev, o16, ln_src_dev, ln_g_dev, ln_b_dev, ln_eps, ln_out_dev, st);
+  return launch_gemm<EPI>(mw, mx, nt, M, N, K, bias_dev, residual_dev, out_f32_dev, o16, st);
+}
+
+extern "C" int mmr_debug_enc_gemm(int32_t epi, int32_t nt, int32_t fold_ln, int32_t M, int32_t N, int32_t K, const void* x_dev,
+                                  const float* ln_src_dev, const float* ln_g_dev, const float* ln_b_dev, float ln_eps,
+                                  float* ln_out_dev, const void* w_dev, const float* bias_dev, const float* residual_dev,
+                                  float* out_f32_dev, void* out_bf16_dev, void* stream) {
+  if (epi < EPI_BIAS_F32 || epi > EPI_QUICKGELU_BF16) return fail(MMR_ERR_INVALID, "unknown epilogue %d", epi);
+  if (nt != 64 && nt != 128 && nt != 256) return fail(MMR_ERR_INVALID, "token tile %d: must be 64, 128 or 256", nt);
+  if (fold_ln != 0 && fold_ln != 1) return fail(MMR_ERR_INVALID, "fold_ln must be 0 or 1");
+  if (M < 1 || M > (1 << 22)) return fail(MMR_ERR_INVALID, "M = %d: must be in [1, 2^22]", M);
+  if (N < ENC_BM || N % ENC_BM != 0 || N > 65535 * ENC_BM) return fail(MMR_ERR_INVALID, "N = %d: must be a positive multiple of 128", N);
+  if (K < 64 || K % 64 != 0) return fail(MMR_ERR_INVALID, "K = %d: must be a positive multiple of 64", K);
+  if (!w_dev || !aligned16(w_dev)) return fail(MMR_ERR_INVALID, "W must be a 16-byte aligned device pointer");
+  if (fold_ln) {
+    if (nt != 64) return fail(MMR_ERR_INVALID, "the LayerNorm-folded GEMM runs on the 64-token tile only (nt = %d)", nt);
+    if (K != 384 && K != 512) return fail(MMR_ERR_INVALID, "the LayerNorm-folded GEMM needs K = 384 or 512 (K = %d)", K);
+    if (epi == EPI_BIAS_RES_F32) return fail(MMR_ERR_INVALID, "the LayerNorm-folded GEMM has no residual epilogue");
+    if (!ln_src_dev || !ln_g_dev || !ln_b_dev) return fail(MMR_ERR_INVALID, "fold_ln needs ln_src, ln_g and ln_b");
+    if (ln_out_dev && static_cast<const void*>(ln_out_dev) == static_cast<const void*>(ln_src_dev))
+      return fail(MMR_ERR_INVALID, "ln_out may not alias ln_src");
+  } else if (!x_dev || !aligned16(x_dev)) {
+    return fail(MMR_ERR_INVALID, "X must be a 16-byte aligned device pointer");
+  }
+  if ((epi == EPI_BIAS_F32 || epi == EPI_BIAS_RES_F32) && !out_f32_dev) return fail(MMR_ERR_INVALID, "epilogue %d needs out_f32", epi);
+  if (epi == EPI_BIAS_RES_F32 && !residual_dev) return fail(MMR_ERR_INVALID, "the residual epilogue needs residual");
+  if ((epi == EPI_GELU_BF16 || epi == EPI_QUICKGELU_BF16) && !out_bf16_dev) return fail(MMR_ERR_INVALID, "epilogue %d needs out_bf16", epi);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (epi) {
+    case EPI_BIAS_F32:
+      return debug_gemm_epi<EPI_BIAS_F32>(nt, fold_ln, M, N, K, x_dev, ln_src_dev, ln_g_dev, ln_b_dev, ln_eps, ln_out_dev, w_dev, bias_dev,
+                                          residual_dev, out_f32_dev, out_bf16_dev, st);
+    case EPI_BIAS_RES_F32:
+      return debug_gemm_epi<EPI_BIAS_RES_F32>(nt, fold_ln, M, N, K, x_dev, ln_src_dev, ln_g_dev, ln_b_dev, ln_eps, ln_out_dev, w_dev,
+                                              bias_dev, residual_dev, out_f32_dev, out_bf16_dev, st);
+    case EPI_GELU_BF16:
+      return debug_gemm_epi<EPI_GELU_BF16>(nt, fold_ln, M, N, K, x_dev, ln_src_dev, ln_g_dev, ln_b_dev, ln_eps, ln_out_dev, w_dev, bias_dev,
+                                           residual_dev, out_f32_dev, out_bf16_dev, st);
+    default:
+      return debug_gemm_epi<EPI_QUICKGELU_BF16>(nt, fold_ln, M, N, K, x_dev, ln_src_dev, ln_g_dev, ln_b_dev, ln_eps, ln_out_dev, w_dev,
+                                                bias_dev, residual_dev, out_f32_dev, out_bf16_dev, st);
+  }
+}
+
+extern "C" int mmr_debug_enc_attention(int32_t tensor_cores, int32_t B, int32_t S, int32_t H, int32_t heads, int32_t causal,
+                                       const float* qkv_dev, const int32_t* mask_dev, void* ctx_dev, void* stream) {
+  if (tensor_cores != 0 && tensor_cores != 1) return fail(MMR_ERR_INVALID, "tensor_cores must be 0 or 1");
+  if (causal != 0 && causal != 1) return fail(MMR_ERR_INVALID, "causal must be 0 or 1");
+  if ((H != 384 && H != 512) || heads < 1 || H % heads != 0 || (H / heads != 32 && H / heads != 64))
+    return fail(MMR_ERR_INVALID, "hidden %d / heads %d: hidden must be 384 or 512 with head dim 32 or 64", H, heads);
+  if (B < 1 || B > 65535) return fail(MMR_ERR_INVALID, "B = %d: must be in [1, 65535]", B);
+  if (S < 1 || S > 512) return fail(MMR_ERR_INVALID, "S = %d: must be in [1, 512]", S);
+  if (!qkv_dev || !ctx_dev || !aligned16(qkv_dev) || !aligned16(ctx_dev))
+    return fail(MMR_ERR_INVALID, "qkv and ctx must be 16-byte aligned device pointers");
+  return launch_attention(tensor_cores != 0, B, S, H, heads, causal, qkv_dev, mask_dev, static_cast<__nv_bfloat16*>(ctx_dev),
+                          static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int mmr_debug_enc_layernorm(int32_t H, int32_t M, const float* x_dev, const float* g_dev, const float* b_dev, float eps,
+                                       float* out_f32_dev, void* out_bf16_dev, void* stream) {
+  if (H != 384 && H != 512) return fail(MMR_ERR_INVALID, "H = %d: must be 384 or 512", H);
+  if (M < 1 || M > (1 << 22)) return fail(MMR_ERR_INVALID, "M = %d: must be in [1, 2^22]", M);
+  if (!x_dev || !g_dev || !b_dev) return fail(MMR_ERR_INVALID, "NULL argument");
+  if (!out_f32_dev && !out_bf16_dev) return fail(MMR_ERR_INVALID, "no output: out_f32 and out_bf16 are both NULL");
+  const int wpb = 8;   // forward_t's rows_grid / rows_block
+  const dim3 grid((M + wpb - 1) / wpb), block(wpb * 32);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  __nv_bfloat16* o16 = static_cast<__nv_bfloat16*>(out_bf16_dev);
+  if (H == 384)
+    CUDA_TRY(launch_pdl(layernorm_kernel<384>, grid, block, 0, st, x_dev, g_dev, b_dev, eps, M, out_f32_dev, o16));
+  else
+    CUDA_TRY(launch_pdl(layernorm_kernel<512>, grid, block, 0, st, x_dev, g_dev, b_dev, eps, M, out_f32_dev, o16));
+  mmr_g_launches++;
+  return MMR_OK;
 }

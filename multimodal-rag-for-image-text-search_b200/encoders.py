@@ -80,6 +80,17 @@ def hf_clip_text_weights(model) -> Dict[str, torch.Tensor]:
     return out
 
 
+def _check_supported(cfg, acts) -> None:
+    """The kernels implement erf-GELU (BERT), quick-GELU (CLIP) and absolute position embeddings only: any other model
+    would run with the wrong math and no error."""
+    act = getattr(cfg, "hidden_act", None)
+    if not isinstance(act, str) or act not in acts:
+        raise ValueError(f"hidden_act {act!r} is not supported by the device encoders (expected {' or '.join(sorted(acts))})")
+    pos = getattr(cfg, "position_embedding_type", "absolute")
+    if pos != "absolute":
+        raise ValueError(f"position_embedding_type {pos!r} is not supported by the device encoders (expected 'absolute')")
+
+
 class DeviceEncoder:
     """One transformer (MiniLM / CLIP text / cross-encoder) resident on a B200, driven through mmr_encoder_*."""
 
@@ -102,6 +113,7 @@ class DeviceEncoder:
     @classmethod
     def from_hf_bert(cls, model, device: Any = "cuda:0", cross: Optional[bool] = None) -> "DeviceEncoder":
         cfg = model.config
+        _check_supported(cfg, {"gelu"})
         weights = hf_bert_weights(model)
         cross = ("cls_w" in weights) if cross is None else cross
         enc = cls("cross" if cross else "minilm", vocab_size=cfg.vocab_size, hidden=cfg.hidden_size,
@@ -114,6 +126,7 @@ class DeviceEncoder:
     @classmethod
     def from_hf_clip(cls, model, device: Any = "cuda:0") -> "DeviceEncoder":
         cfg = getattr(model.config, "text_config", model.config)
+        _check_supported(cfg, {"quick_gelu"})
         weights = hf_clip_text_weights(model)
         enc = cls("clip_text", vocab_size=cfg.vocab_size, hidden=cfg.hidden_size, layers=cfg.num_hidden_layers,
                   heads=cfg.num_attention_heads, intermediate=cfg.intermediate_size,

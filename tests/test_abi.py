@@ -59,3 +59,65 @@ def test_no_cpu_fallback():
         pkg.B200Store()
     with pytest.raises(pkg.NativeError):
         pkg.ResidentIndex(torch.zeros(8, 512, dtype=torch.bfloat16))
+
+
+def test_encoder_debug_hooks_reject_bad_arguments():
+    """mmr_debug_enc_gemm / _attention / _layernorm check every argument before any CUDA call: MMR_ERR_INVALID and a message
+    naming what is wrong (the buffers below are never dereferenced)."""
+    lib = native.lib()
+    buf = (C.c_float * 64)()
+    p = C.addressof(buf)                                   # 16-byte aligned, stands in for a device buffer
+    odd = p + 2
+
+    def gemm(epi=0, nt=64, fold=0, M=64, N=128, K=64, x=p, src=None, g=None, b=None, ln_out=None, w=p, res=None, o32=p, o16=p):
+        return lib.mmr_debug_enc_gemm(epi, nt, fold, M, N, K, x, src, g, b, 1e-5, ln_out, w, None, res, o32, o16, None)
+
+    cases = [
+        (dict(epi=4), b"epilogue"), (dict(epi=-1), b"epilogue"),
+        (dict(nt=32), b"token tile"), (dict(nt=512), b"token tile"),
+        (dict(fold=2), b"fold_ln"),
+        (dict(M=0), b"M = 0"),
+        (dict(N=192), b"N = 192"), (dict(N=0), b"N = 0"),
+        (dict(K=96), b"K = 96"), (dict(K=0), b"K = 0"),
+        (dict(w=None), b"W must"), (dict(w=odd), b"W must"),
+        (dict(x=None), b"X must"), (dict(x=odd), b"X must"),
+        (dict(fold=1, nt=128, K=384, src=p, g=p, b=p), b"64-token tile"),
+        (dict(fold=1, K=1536, src=p, g=p, b=p), b"K = 384 or 512"),
+        (dict(fold=1, K=384, epi=1, src=p, g=p, b=p, res=p), b"no residual"),
+        (dict(fold=1, K=384, g=p, b=p), b"ln_src"),
+        (dict(fold=1, K=384, src=p, b=p), b"ln_g"),
+        (dict(fold=1, K=384, src=p, g=p), b"ln_b"),
+        (dict(fold=1, K=384, src=p, g=p, b=p, ln_out=p), b"alias"),
+        (dict(epi=0, o32=None), b"out_f32"),
+        (dict(epi=1, res=p, o32=None), b"out_f32"),
+        (dict(epi=1, res=None), b"residual"),
+        (dict(epi=2, o16=None), b"out_bf16"),
+        (dict(epi=3, o16=None), b"out_bf16"),
+    ]
+    for kw, words in cases:
+        assert gemm(**kw) == 1, kw                          # MMR_ERR_INVALID
+        assert words in lib.mmr_last_error(), (kw, lib.mmr_last_error())
+
+    def att(tc=0, B=1, S=64, H=384, heads=12, causal=0, qkv=p, mask=None, ctx=p):
+        return lib.mmr_debug_enc_attention(tc, B, S, H, heads, causal, qkv, mask, ctx, None)
+
+    cases = [
+        (dict(tc=2), b"tensor_cores"), (dict(causal=-1), b"causal"),
+        (dict(H=768), b"hidden 768"), (dict(heads=0), b"heads 0"), (dict(heads=4), b"heads 4"), (dict(heads=5), b"heads 5"),
+        (dict(B=0), b"B = 0"), (dict(S=0), b"S = 0"), (dict(S=513), b"S = 513"),
+        (dict(qkv=None), b"qkv and ctx"), (dict(ctx=None), b"qkv and ctx"), (dict(qkv=odd), b"qkv and ctx"),
+    ]
+    for kw, words in cases:
+        assert att(**kw) == 1, kw
+        assert words in lib.mmr_last_error(), (kw, lib.mmr_last_error())
+    # head dim 64 on the fp32 kernel ends at 330 tokens (MMR_ERR_UNSUPPORTED, before any CUDA call)
+    assert att(S=331, heads=6) == 3 and b"fp32 attention kernel" in lib.mmr_last_error()
+    assert att(S=512, H=512, heads=8) == 3 and b"330 tokens at most" in lib.mmr_last_error()
+
+    def ln(H=384, M=4, x=p, g=p, b=p, o32=p, o16=None):
+        return lib.mmr_debug_enc_layernorm(H, M, x, g, b, 1e-5, o32, o16, None)
+
+    for kw, words in [(dict(H=256), b"H = 256"), (dict(M=0), b"M = 0"), (dict(x=None), b"NULL"), (dict(g=None), b"NULL"),
+                      (dict(b=None), b"NULL"), (dict(o32=None), b"no output")]:
+        assert ln(**kw) == 1, kw
+        assert words in lib.mmr_last_error(), (kw, lib.mmr_last_error())

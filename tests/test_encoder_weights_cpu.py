@@ -38,3 +38,24 @@ def test_no_device_no_encoder():
         pytest.skip("CUDA present")
     with pytest.raises(Exception):
         enc_mod.DeviceEncoder("minilm", vocab_size=10, hidden=384, layers=1, heads=12, intermediate=1536, max_positions=8)
+
+
+def test_unsupported_activation_or_position_type_is_refused_before_the_library():
+    """The kernels implement erf-GELU (BERT), quick-GELU (CLIP) and absolute positions only; another model must be refused
+    with ValueError before any library call (no GPU needed: the check runs first)."""
+    import pytest
+    from transformers import BertConfig, BertModel, CLIPTextConfig, CLIPTextModelWithProjection
+    small = dict(vocab_size=100, hidden_size=384, num_hidden_layers=1, num_attention_heads=12, intermediate_size=1536,
+                 max_position_embeddings=64)
+    for kw, words in ((dict(hidden_act="gelu_new"), "hidden_act"), (dict(hidden_act="relu"), "hidden_act"),
+                      (dict(position_embedding_type="relative_key"), "position_embedding_type"),
+                      (dict(position_embedding_type="relative_key_query"), "position_embedding_type")):
+        with pytest.raises(ValueError, match=words):
+            enc_mod.DeviceEncoder.from_hf_bert(BertModel(BertConfig(**small, **kw), add_pooling_layer=False))
+    for act in ("gelu", "gelu_new"):
+        with pytest.raises(ValueError, match="hidden_act"):
+            enc_mod.DeviceEncoder.from_hf_clip(CLIPTextModelWithProjection(CLIPTextConfig(num_hidden_layers=1, vocab_size=100,
+                                                                                           hidden_act=act)))
+    # the supported configs pass the check (and then need the library and a device)
+    enc_mod._check_supported(BertConfig(**small), {"gelu"})
+    enc_mod._check_supported(CLIPTextConfig(num_hidden_layers=1), {"quick_gelu"})

@@ -137,7 +137,12 @@ def test_cross_encoder_logits_match_fp32_torch(enc_mod):
     model = _round_linear_weights(_spread(BertForSequenceClassification(cfg)))
     enc = enc_mod.DeviceEncoder.from_hf_bert(model)
     assert enc.kind == "cross" and enc.out_dim == 1
-    for b, s in ((8, 64), (3, 300), (16, 128), (72, 64)):      # token tiles of 64, 128 and 256
+    _check_cross_encoder(enc, model, ((8, 64), (3, 300), (16, 128), (72, 64)))      # token tiles of 64, 128 and 256
+    enc.close()
+
+
+def _check_cross_encoder(enc, model, shapes):
+    for b, s in shapes:
         g = torch.Generator().manual_seed(s)
         ids = torch.randint(1000, 30000, (b, s), generator=g)
         lens = torch.randint(s // 2, s + 1, (b,), generator=g)
@@ -153,6 +158,190 @@ def test_cross_encoder_logits_match_fp32_torch(enc_mod):
             for j in range(b):
                 if want[i] - want[j] > 2 * bound.max():
                     assert got[i] > got[j], "rerank order differs from fp32 torch beyond the tolerance"
+
+
+@pytest.mark.parametrize("hidden,heads", ((384, 6), (512, 8)))
+def test_cross_encoder_with_head_dim_64_takes_512_tokens(enc_mod, hidden, heads):
+    """A head-dim-64 cross-encoder (hidden 384 / 6 heads, 512 / 8 heads: attention_mma_kernel<64>, and at 512 the BERT branch
+    of forward_t<512>, embed_kernel<512> with token types, cross_head_kernel with 512 threads) up to the 512 tokens a rerank
+    passage may have.  The tensor-core attention needs 149,504 bytes of shared memory at 512 tokens; the fp32 kernel's
+    limit (330 tokens at head dim 64) does not apply to it."""
+    from transformers import BertConfig, BertForSequenceClassification
+    torch.manual_seed(hidden + heads)
+    cfg = BertConfig(vocab_size=30522, hidden_size=hidden, num_hidden_layers=6, num_attention_heads=heads,
+                     intermediate_size=4 * hidden, max_position_embeddings=512, num_labels=1)
+    model = _round_linear_weights(_spread(BertForSequenceClassification(cfg)))
+    enc = enc_mod.DeviceEncoder.from_hf_bert(model)
+    _check_cross_encoder(enc, model, ((8, 64), (3, 331), (2, 512)))
+    enc.close()
+
+
+def test_minilm_at_hidden_512_matches_fp32_torch(enc_mod):
+    """A MiniLM-kind encoder (BertModel, mean pooling) at hidden 512 / 8 heads: forward_t<512> through the BERT branch and the
+    fp32 attention at head dim 64, up to its 330-token limit; 331 tokens are refused with a message."""
+    from transformers import BertConfig, BertModel
+    torch.manual_seed(3)
+    cfg = BertConfig(vocab_size=30522, hidden_size=512, num_hidden_layers=4, num_attention_heads=8, intermediate_size=2048,
+                     max_position_embeddings=512)
+    model = _round_linear_weights(_spread(BertModel(cfg, add_pooling_layer=False)))
+    enc = enc_mod.DeviceEncoder.from_hf_bert(model)
+    assert enc.kind == "minilm" and enc.out_dim == 512
+    for b, s in ((1, 12), (5, 40), (33, 7), (2, 330)):
+        g = torch.Generator().manual_seed(b * 1000 + s)
+        ids = torch.randint(1000, 30000, (b, s), generator=g)
+        lens = torch.randint(max(1, s // 3), s + 1, (b,), generator=g)
+        lens[0] = s
+        mask = (torch.arange(s)[None, :] < lens[:, None]).long()
+        types = (torch.arange(s)[None, :] >= (lens[:, None] // 2)).long() * mask
+        got = enc.forward_ids(ids.numpy(), mask.numpy(), types.numpy()).cpu()
+        want = _bert_reference(model, ids, mask, types)
+        assert (got - want).abs().max().item() <= TOL, (b, s, (got - want).abs().max().item())
+    with pytest.raises(enc_mod.N.NativeError, match="330 tokens at most"):
+        enc.forward_ids(np.ones((1, 331), np.int64))
+    enc.close()
+
+
+def _clip_ids(b, s, seed, eos=49407):
+    """BOS, random tokens, EOS closing every sequence and repeated as padding (the CLIP tokenizer's layout)."""
+    g = torch.Generator().manual_seed(seed)
+    ids = torch.randint(1000, 40000, (b, s), generator=g)
+    ids[:, 0] = 49406
+    lens = torch.randint(min(3, s), s + 1, (b,), generator=g)
+    lens[0] = s
+    mask = (torch.arange(s)[None, :] < lens[:, None]).long()
+    for i in range(b):
+        ids[i, lens[i] - 1:] = eos
+    return ids, mask
+
+
+def _clip_reference(model, ids, mask):
+    with torch.no_grad():
+        return torch.nn.functional.normalize(model(input_ids=ids, attention_mask=mask).text_embeds, dim=1)
+
+
+@pytest.mark.parametrize("variant", ("legacy_eos", "projection_256"))
+def test_clip_text_tower_variants_match_fp32_torch(enc_mod, variant):
+    """eos_token_id = 2 (what openai/clip-vit-base-patch32 ships) selects HF's legacy pooling rule, the position of the
+    largest token id; no token here is 2, so the first-occurrence rule would pool position 0 instead.  projection_dim 256
+    < hidden 512 leaves half the head's threads without a projection output."""
+    from transformers import CLIPTextConfig, CLIPTextModelWithProjection
+    torch.manual_seed(4)
+    cfg = CLIPTextConfig(num_hidden_layers=4, **({"eos_token_id": 2} if variant == "legacy_eos" else {"projection_dim": 256}))
+    model = _round_linear_weights(_spread(CLIPTextModelWithProjection(cfg), 2.0))
+    enc = enc_mod.DeviceEncoder.from_hf_clip(model)
+    assert enc.out_dim == (512 if variant == "legacy_eos" else 256)
+    for b, s in ((1, 9), (6, 25), (40, 77)):
+        ids, mask = _clip_ids(b, s, seed=s)
+        want = _clip_reference(model, ids, mask)
+        got = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+        assert got.shape == want.shape
+        assert (got - want).abs().max().item() <= TOL, (variant, b, s, (got - want).abs().max().item())
+    enc.close()
+
+
+def test_clip_on_the_tensor_core_attention_matches_fp32_torch(enc_mod):
+    """MMR_ENC_ATT_MMA=2 runs every model's attention on attention_mma_kernel from 96 tokens on: here the causal branch,
+    against HF at S = 100.  Bound: the shipped path rounds one attention quantity to bf16 (the context, 2^-9 relative) and
+    stays within TOL.  The tensor-core kernel also rounds q, k, v and the softmax weights P to bf16: four more roundings of
+    2^-9, and the q / k roundings move each score s by up to 2^-8 |s|, i.e. each weight by up to 2^-8 |s| relative, with
+    |s| <= 4 for the scaled weights here.  That is at most 1 + 4 + 2 * 4 = 13 times the shipped path's attention rounding;
+    the rest of the network (GEMM inputs, LayerNorms) is unchanged, so 13 * TOL bounds the embedding error."""
+    from transformers import CLIPTextConfig, CLIPTextModelWithProjection
+    native = importlib.import_module(PKG + "._native")
+    torch.manual_seed(6)
+    model = _round_linear_weights(_spread(CLIPTextModelWithProjection(CLIPTextConfig(num_hidden_layers=3,
+                                                                                      max_position_embeddings=128)), 2.0))
+    enc = enc_mod.DeviceEncoder.from_hf_clip(model)
+    ids, mask = _clip_ids(4, 100, seed=100)
+    want = _clip_reference(model, ids, mask)
+    try:
+        fp32 = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+        native.set_option("MMR_ENC_ATT_MMA", "2")
+        got = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+    finally:
+        native.set_option("MMR_ENC_ATT_MMA", None)
+        enc.close()
+    assert not torch.equal(got, fp32), "MMR_ENC_ATT_MMA=2 must switch the attention kernel"
+    assert (fp32 - want).abs().max().item() <= TOL
+    assert (got - want).abs().max().item() <= 13 * TOL, (got - want).abs().max().item()
+
+
+def test_layernorm_folded_into_the_gemm_matches_the_separate_kernel_for_clip(enc_mod):
+    """The CLIP (pre-LN) side of the folded LayerNorm: LN1 in front of QKV and LN2 in front of FC1 (quick-GELU epilogue),
+    both with ln_out = NULL.  Bit-identical embeddings to the layernorm_kernel path, two launches fewer per layer."""
+    from transformers import CLIPTextConfig, CLIPTextModelWithProjection
+    native = importlib.import_module(PKG + "._native")
+    torch.manual_seed(8)
+    layers = 4
+    model = _round_linear_weights(_spread(CLIPTextModelWithProjection(CLIPTextConfig(num_hidden_layers=layers)), 2.0))
+    enc = enc_mod.DeviceEncoder.from_hf_clip(model)
+    try:
+        for b, s in ((1, 9), (1, 16), (4, 40), (9, 77)):     # 9 / 16 / 160 / 693 tokens: 1, 1, 3 and 11 token tiles
+            ids, mask = _clip_ids(b, s, seed=b * s)
+            want = _clip_reference(model, ids, mask)
+            outs = {}
+            for mode in ("0", "2"):
+                native.set_option("MMR_ENC_FUSE_LN", mode)
+                n0 = native.lib().mmr_launch_count()
+                outs[mode] = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+                outs[mode + "n"] = native.lib().mmr_launch_count() - n0
+                assert (outs[mode] - want).abs().max().item() <= TOL, (mode, b, s)
+            assert outs["2n"] == outs["0n"] - 2 * layers, (outs["0n"], outs["2n"])
+            assert torch.equal(outs["0"], outs["2"]), (b, s)
+    finally:
+        native.set_option("MMR_ENC_FUSE_LN", None)
+        enc.close()
+
+
+def _token_tile(M, N, sms):
+    """enc_token_tile_for (csrc/mmr_encoder.cu): the tile by token count, halved while the grid would leave SMs idle."""
+    nt = 64 if M <= 1024 else (128 if M <= 4096 else 256)
+    while nt > 64 and (N // 128) * ((M + nt - 1) // nt) < (1 if nt == 256 else 2) * sms:
+        nt //= 2
+    return nt
+
+
+def _sm_count(native):
+    import ctypes as C
+    n = C.c_int(0)
+    native.check(native.lib().mmr_device_sm_count(0, C.byref(n)))
+    return n.value
+
+
+def test_query_embedding_does_not_depend_on_the_micro_batch_token_tile(enc_mod, bert):
+    """A query's embedding is bit-identical alone and inside a micro-batch large enough to move the QKV / FFN1 GEMMs off
+    the 64-token tile (MiniLM 128 x 40 tokens; CLIP 40 x 77 and 128 x 77).  The tiles are computed here with the library's
+    rule from the device's SM count, and the test requires that a tile other than 64 really ran."""
+    from transformers import CLIPTextConfig, CLIPTextModelWithProjection
+    native = importlib.import_module(PKG + "._native")
+    sms = _sm_count(native)
+    g = torch.Generator().manual_seed(21)
+    enc = enc_mod.DeviceEncoder.from_hf_bert(bert)
+    q = torch.randint(1000, 30000, (13,), generator=g)
+    alone = enc.forward_ids(q[None].numpy()).cpu()
+    b, s = 128, 40
+    assert _token_tile(b * s, min(3 * 384, 1536), sms) != 64
+    ids = torch.randint(1000, 30000, (b, s), generator=g)
+    lens = torch.randint(5, s + 1, (b,), generator=g)
+    ids[77, :13], lens[77] = q, 13
+    mask = (torch.arange(s)[None, :] < lens[:, None]).long()
+    batch = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+    assert torch.equal(batch[77], alone[0]), float((batch[77] - alone[0]).abs().max())
+    enc.close()
+
+    torch.manual_seed(9)
+    clip = _round_linear_weights(_spread(CLIPTextModelWithProjection(CLIPTextConfig(num_hidden_layers=4)), 2.0))
+    enc = enc_mod.DeviceEncoder.from_hf_clip(clip)
+    qc, _ = _clip_ids(1, 11, seed=5)
+    alone = enc.forward_ids(qc.numpy()).cpu()
+    for b in (40, 128):
+        assert _token_tile(b * 77, min(3 * 512, 2048), sms) != 64, (b, sms)
+        ids, mask = _clip_ids(b, 77, seed=b)
+        ids[b // 2] = 49407
+        ids[b // 2, :11] = qc[0]
+        mask[b // 2] = (torch.arange(77) < 11).long()
+        batch = enc.forward_ids(ids.numpy(), mask.numpy()).cpu()
+        assert torch.equal(batch[b // 2], alone[0]), (b, float((batch[b // 2] - alone[0]).abs().max()))
     enc.close()
 
 
