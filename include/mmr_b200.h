@@ -235,6 +235,9 @@ int mmr_fuse_f64(const double* text_scores_dev, const int32_t* text_count_dev, c
  *                      LayerNorm -> text_projection -> L2 norm -> [B, proj_dim]   (app/ml/embeddings.py:94-105)
  *   MMR_ENC_CROSS      CrossEncoder.predict: the same BERT + pooler (tanh) + 1-logit classifier -> [B] raw logits
  *                      (app/ml/retrieve.py:29-38,146; cross-encoder/ms-marco-MiniLM-L-6-v2)
+ *   MMR_ENC_CLIP_VISION  embed_images_batch, the ingest side: CLIP vision tower (ViT-B/32) -> [B, proj_dim]
+ *                      (app/ml/embeddings.py:73-91); created with mmr_encoder_create_vision, run with
+ *                      mmr_encoder_forward_pixels (below)
  * Tokenisation stays with the caller (HF tokenizers need the vocabulary files): the calls take token ids.
  * Weights are handed over once, by name, as fp32 device arrays in nn.Linear layout ([out, in]); GEMM weights are kept
  * as bf16, everything else as fp32:
@@ -271,6 +274,32 @@ int mmr_encoder_forward(mmr_encoder* encoder, const int32_t* input_ids_host, con
                         const int32_t* token_type_host, int32_t B, int32_t S, float* out_dev, void* stream);
 
 /*
+ * CLIP vision tower (HF CLIPVisionModelWithProjection; what CLIPModel.get_image_features computes): pixels -> patch
+ * embedding (Conv2d, stride = kernel = patch_size, no bias, run as patchify + one GEMM) -> class token + position
+ * embeddings -> pre-LayerNorm -> `layers` pre-LN quick-GELU layers (no mask, not causal) -> class token -> final LayerNorm
+ * (HF post_layernorm) -> visual_projection -> L2 norm.  Image preprocessing (decode, resize, crop, normalise) stays with the
+ * caller (HF CLIPImageProcessor), as tokenisation does for the text encoders.
+ * Config limits, checked before any CUDA call (MMR_ERR_INVALID / MMR_ERR_UNSUPPORTED with a message): hidden 768 with head
+ * dim 64; image_size a multiple of patch_size; channels * patch_size^2 a multiple of 64; intermediate a multiple of 128;
+ * (image_size / patch_size)^2 + 1 <= 330 tokens (the fp32 attention at head dim 64: ViT-B/32 has 50, ViT-B/16 197);
+ * 0 < proj_dim <= hidden.
+ * Weights by name through mmr_encoder_set_weight: patch_w ([hidden, channels * patch_size^2]: the Conv2d weight
+ * [hidden, C, P, P] flattened, kept as bf16) cls_emb ([hidden]) pos_emb ([tokens, hidden]) pre_ln_w pre_ln_b |
+ * L<i>.* exactly as for MMR_ENC_CLIP_TEXT | final_ln_w final_ln_b proj_w ([proj_dim, hidden]).
+ * mmr_encoder_forward on a vision encoder, and mmr_encoder_forward_pixels on a text encoder, fail with MMR_ERR_INVALID.
+ */
+enum { MMR_ENC_CLIP_VISION = 3 };
+typedef struct mmr_vision_config {
+  int32_t hidden, layers, heads, intermediate, image_size, patch_size, channels, proj_dim;
+  float ln_eps;
+} mmr_vision_config;
+int mmr_encoder_create_vision(int device, const mmr_vision_config* config, mmr_encoder** out);
+/* One forward pass for B >= 1 images: pixels_dev fp32 [B, channels, image_size, image_size] (NCHW, what
+ * CLIPImageProcessor returns) on the encoder's device; out_dev [B, proj_dim] fp32 unit-norm rows, directly usable as
+ * mmr_search queries or as rows for mmr_convert_rows_f32.  Calls on one encoder take turns, as mmr_encoder_forward's do. */
+int mmr_encoder_forward_pixels(mmr_encoder* encoder, const float* pixels_dev, int32_t B, float* out_dev, void* stream);
+
+/*
  * Validation hook for the tensor-core path (K2): raw cosine scores of B queries against rows
  * [row_begin, row_end) as computed by the tcgen05 contraction (bf16 queries x bf16 rows, fp32 accumulate),
  * written to out_scores_dev[b * out_ld + (row - row_begin)].  workspace as for mmr_search(B, k = 10).
@@ -296,6 +325,11 @@ int mmr_debug_umma_scores(const mmr_index* index, const float* queries_dev, int3
  *       key) or NULL; causal hides keys after the query row.  Sequence limits as for mmr_encoder_forward.
  *   mmr_debug_enc_layernorm  layernorm_kernel<H>, H 384 or 512: rows of x fp32 [M, H] -> out_f32 (may equal x) and / or
  *       out_bf16 bf16 [M, H].
+ *   mmr_debug_enc_patch_embed  the vision front end, three launches as mmr_encoder_forward_pixels makes them (H 768): pixels
+ *       fp32 [B, C, image_size, image_size] -> patch16 bf16 [B * NP, C * patch^2] (the patch matrix: NP = (image_size /
+ *       patch)^2 patches in row-major order, columns in (c, kh, kw) order, values bf16(pixel)) -> patch_out fp32 [B * NP, H]
+ *       = patch16 . patch_w^T (patch_w bf16 [H, C * patch^2]) -> x fp32 [B * (NP + 1), H]: per image, row 0 = cls + pos[0],
+ *       row 1 + p = patch_out[p] + pos[1 + p], each then LayerNorm(ln_g, ln_b, ln_eps).  patch16 and patch_out are written.
  */
 int mmr_debug_enc_gemm(int32_t epi, int32_t nt, int32_t fold_ln, int32_t M, int32_t N, int32_t K, const void* x_dev,
                        const float* ln_src_dev, const float* ln_g_dev, const float* ln_b_dev, float ln_eps, float* ln_out_dev,
@@ -305,6 +339,10 @@ int mmr_debug_enc_attention(int32_t tensor_cores, int32_t B, int32_t S, int32_t 
                             const float* qkv_dev, const int32_t* mask_dev, void* ctx_dev, void* stream);
 int mmr_debug_enc_layernorm(int32_t H, int32_t M, const float* x_dev, const float* g_dev, const float* b_dev, float eps,
                             float* out_f32_dev, void* out_bf16_dev, void* stream);
+int mmr_debug_enc_patch_embed(int32_t H, int32_t C, int32_t image_size, int32_t patch, int32_t B, const float* pixels_dev,
+                              const void* patch_w_dev, const float* cls_dev, const float* pos_dev, const float* ln_g_dev,
+                              const float* ln_b_dev, float ln_eps, void* patch16_dev, float* patch_out_dev, float* x_dev,
+                              void* stream);
 
 /* Introspection used by bench.py / tests: launches issued by this library since load, device facts. */
 int64_t mmr_launch_count(void);

@@ -48,12 +48,15 @@ SYMBOLS = [
     ("mmr_encoder_out_dim", C.c_int, [_p]),
     ("mmr_encoder_set_weight", C.c_int, [_p, C.c_char_p, _p, _i64, _p]),
     ("mmr_encoder_forward", C.c_int, [_p, _p, _p, _p, _i32, _i32, _p, _p]),
+    ("mmr_encoder_create_vision", C.c_int, [C.c_int, _p, C.POINTER(_p)]),
+    ("mmr_encoder_forward_pixels", C.c_int, [_p, _p, _i32, _p, _p]),
     ("mmr_fuse", C.c_int, [_p, _p, _i32, _p, _p, _i32, _i32, _i32, _f64, _p, _p, _p, _p, _p, _p]),
     ("mmr_fuse_f64", C.c_int, [_p, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _f64, _p, _p, _p, _p]),
     ("mmr_debug_umma_scores", C.c_int, [_p, _p, _i32, _i64, _i64, _p, _i64, _p, _sz, _p]),
     ("mmr_debug_enc_gemm", C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, C.c_float, _p, _p, _p, _p, _p, _p, _p]),
     ("mmr_debug_enc_attention", C.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p]),
     ("mmr_debug_enc_layernorm", C.c_int, [_i32, _i32, _p, _p, _p, C.c_float, _p, _p, _p]),
+    ("mmr_debug_enc_patch_embed", C.c_int, [_i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, C.c_float, _p, _p, _p, _p]),
     ("mmr_launch_count", _i64, []),
     ("mmr_device_sm_count", C.c_int, [C.c_int, C.POINTER(C.c_int)]),
     ("mmr_last_kernel", C.c_int, []),
@@ -61,7 +64,7 @@ SYMBOLS = [
 ]
 
 
-MMR_ENC_MINILM, MMR_ENC_CLIP_TEXT, MMR_ENC_CROSS = 0, 1, 2
+MMR_ENC_MINILM, MMR_ENC_CLIP_TEXT, MMR_ENC_CROSS, MMR_ENC_CLIP_VISION = 0, 1, 2, 3
 
 
 class EncoderConfig(C.Structure):
@@ -69,6 +72,12 @@ class EncoderConfig(C.Structure):
     _fields_ = [("kind", _i32), ("vocab_size", _i32), ("hidden", _i32), ("layers", _i32), ("heads", _i32),
                 ("intermediate", _i32), ("max_positions", _i32), ("type_vocab", _i32), ("proj_dim", _i32),
                 ("eos_token_id", _i32), ("ln_eps", C.c_float)]
+
+
+class VisionConfig(C.Structure):
+    """mmr_vision_config (include/mmr_b200.h)."""
+    _fields_ = [("hidden", _i32), ("layers", _i32), ("heads", _i32), ("intermediate", _i32), ("image_size", _i32),
+                ("patch_size", _i32), ("channels", _i32), ("proj_dim", _i32), ("ln_eps", C.c_float)]
 
 
 class NativeError(RuntimeError):

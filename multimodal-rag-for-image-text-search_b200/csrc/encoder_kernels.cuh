@@ -3,7 +3,11 @@
 //   embed_query_for_images  (CLIP ViT-B/32 text tower: 12 pre-LN layers, hidden 512, causal, EOS pooling, projection, L2 norm)
 //                                                                                              reference app/ml/embeddings.py:94-105
 //   CrossEncoder.predict    (ms-marco-MiniLM-L-6: the same BERT + pooler + 1-logit classifier) reference app/ml/retrieve.py:132-155
-// so that a query is born on the GPU and feeds mmr_search directly.
+// so that a query is born on the GPU and feeds mmr_search directly, and the one model of the ingest side
+//   embed_images_batch      (CLIP ViT-B/32 vision tower: patchify + patch GEMM, class token, pre-LayerNorm, the same 12 pre-LN
+//                            layers at hidden 768, not causal, class-token pooling, projection, L2 norm)
+//                                                                                              reference app/ml/embeddings.py:73-91
+// so that an image's index row is made by the same kernels as the query it is searched with.
 //
 // These models are small and latency-bound (a query is 8-40 tokens; 21 / 75 MB of bf16 weights stay in L2), so the
 // kernels are shaped for short sequences and batch <= 128:
@@ -355,6 +359,47 @@ __global__ void layernorm_kernel(const float* __restrict__ x, const float* __res
     if (out_f32) out_f32[size_t(t) * H + c] = y[i];
     if (out_bf16) out_bf16[size_t(t) * H + c] = __float2bfloat16_rn(y[i]);
   }
+}
+
+// ---------------------------------------------------------------------------------------------- CLIP vision front end
+// Patchify: pixels fp32 [B, C, S_img, S_img] (NCHW) -> the patch GEMM's token operand bf16 [B * NP, C * P * P], NP = (S_img / P)^2
+// patches in row-major order (HF: conv output flattened over (h, w)), columns in (c, kh, kw) order = the flattened Conv2d
+// weight [H, C, P, P].  Values are only rounded: out = bf16_rn(pixel).  One CTA per patch row; consecutive threads take
+// consecutive columns, i.e. consecutive pixels of an image row (coalesced reads and writes).
+__global__ void patchify_kernel(const float* __restrict__ pixels, int C, int S_img, int P, __nv_bfloat16* __restrict__ out) {
+  pdl_chain_prologue();
+  const int gw = S_img / P, np = gw * gw, cols = C * P * P;
+  const int row = blockIdx.x, b = row / np, p = row % np;
+  const int ph = p / gw, pw = p % gw;
+  const float* img = pixels + size_t(b) * C * S_img * S_img;
+  for (int col = threadIdx.x; col < cols; col += blockDim.x) {
+    const int c = col / (P * P), r = col % (P * P), kh = r / P, kw = r % P;
+    out[size_t(row) * cols + col] = __float2bfloat16_rn(img[(size_t(c) * S_img + ph * P + kh) * S_img + pw * P + kw]);
+  }
+}
+
+// CLIP vision embeddings + pre-LayerNorm, warp per token: token 0 of an image = cls + pos[0], token 1 + p = patch_out[p] +
+// pos[1 + p] (patch_out fp32 [B * (T - 1), H] = the patch GEMM's output), then LN(pre_ln_g, pre_ln_b) -> the fp32 residual
+// stream (HF's pre_layrnorm output is the encoder's input hidden state).  T = tokens per image.
+template <int H>
+__global__ void vision_embed_kernel(const float* __restrict__ patch_out, const float* __restrict__ cls, const float* __restrict__ pos,
+                                    const float* __restrict__ ln_g, const float* __restrict__ ln_b, float eps, int M, int T,
+                                    float* __restrict__ x_f32) {
+  pdl_chain_prologue();
+  const int lane = threadIdx.x & 31;
+  const int t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (t >= M) return;
+  const int b = t / T, p = t % T;
+  const float* src = p == 0 ? cls : patch_out + (size_t(b) * (T - 1) + p - 1) * H;
+  float x[H / 32], y[H / 32];
+#pragma unroll
+  for (int i = 0; i < H / 32; ++i) {
+    const int c = i * 32 + lane;
+    x[i] = src[c] + pos[size_t(p) * H + c];
+  }
+  warp_layernorm<H>(x, ln_g, ln_b, eps, lane, y);
+#pragma unroll
+  for (int i = 0; i < H / 32; ++i) x_f32[size_t(t) * H + i * 32 + lane] = y[i];
 }
 
 // ---------------------------------------------------------------------------------------------- attention
@@ -728,8 +773,9 @@ __global__ void mean_pool_norm_kernel(const float* __restrict__ x, const int32_t
   out[size_t(b) * H + c] = nrm > 0.f ? e / nrm : e;
 }
 
-// CLIP text head: hidden state at the EOS position -> final LayerNorm -> text_projection (no bias) -> L2 normalisation.
-// blockDim.x == H == projection dim (512).  eos_id == 2 reproduces the legacy argmax(input_ids) rule of HF's CLIP.
+// CLIP head: hidden state at the pooled position -> final LayerNorm -> projection (no bias) -> L2 normalisation.
+// blockDim.x == H >= projection dim P.  Text tower: the EOS position (eos_id == 2 reproduces the legacy argmax(input_ids)
+// rule of HF's CLIP).  Vision tower (ids == nullptr): position 0, the class token.
 __global__ void clip_head_kernel(const float* __restrict__ x, const int32_t* __restrict__ ids, int S, int H, int eos_id,
                                  const float* __restrict__ ln_g, const float* __restrict__ ln_b, float eps,
                                  const float* __restrict__ proj /* [P, H] */, int P, float* __restrict__ out) {
@@ -740,7 +786,9 @@ __global__ void clip_head_kernel(const float* __restrict__ x, const int32_t* __r
   const int b = blockIdx.x, c = threadIdx.x;
   if (c == 0) {
     int pos = 0;
-    if (eos_id == 2) {
+    if (ids == nullptr) {
+      // class token
+    } else if (eos_id == 2) {
       int best = ids[size_t(b) * S];
       for (int t = 1; t < S; ++t)
         if (ids[size_t(b) * S + t] > best) {

@@ -38,12 +38,17 @@ bool make_map(CUtensorMap* map, const void* base, int64_t rows, int cols, int bo
 
 struct mmr_encoder {
   int device = 0;
-  mmr_encoder_config cfg{};
+  mmr_encoder_config cfg{};     // vision: kind MMR_ENC_CLIP_VISION, max_positions = tokens per image, no vocabulary
+  mmr_vision_config vcfg{};
+  int patch_cols = 0;           // vision: C * P * P, the patch GEMM's K
   int out_dim = 0;
   std::mutex mu;
   std::vector<LayerW> layers;
   float *word = nullptr, *pos = nullptr, *type_emb = nullptr, *emb_ln_w = nullptr, *emb_ln_b = nullptr;
   float *final_ln_w = nullptr, *final_ln_b = nullptr, *proj_w = nullptr;                     // CLIP
+  float *cls_emb = nullptr, *pre_ln_w = nullptr, *pre_ln_b = nullptr;                         // CLIP vision
+  __nv_bfloat16* patch_w = nullptr;                                                           // [H, C * P * P]
+  CUtensorMap m_patch_w;
   float *pool_w = nullptr, *pool_b = nullptr, *cls_w = nullptr, *cls_b = nullptr;            // cross-encoder
   std::vector<void*> owned;
   std::map<std::string, bool> seen;
@@ -53,9 +58,10 @@ struct mmr_encoder {
   __nv_bfloat16 *x16 = nullptr, *ctx16 = nullptr, *h16 = nullptr;
   int32_t *d_ids = nullptr, *d_mask = nullptr, *d_types = nullptr, *h_stage = nullptr;
   CUtensorMap m_x16, m_ctx16, m_h16;
+  CUtensorMap m_patch;                     // vision: the patch matrix [B * NP, C * P * P] bf16, held in h16
   int maps_tokens = -1;
   int maps_narrow = -1;
-  int nt_x = 64, nt_ctx = 64, nt_h = 64;   // token tiles (= box rows) of the activation maps
+  int nt_x = 64, nt_ctx = 64, nt_h = 64, nt_patch = 64;   // token tiles (= box rows) of the activation maps
 };
 
 static int dev_alloc(mmr_encoder* e, void** p, size_t bytes) {
@@ -64,16 +70,9 @@ static int dev_alloc(mmr_encoder* e, void** p, size_t bytes) {
   return MMR_OK;
 }
 
-extern "C" int mmr_encoder_create(int device, const mmr_encoder_config* cfg, mmr_encoder** out) {
-  if (!out || !cfg) return fail(MMR_ERR_INVALID, "NULL argument");
-  *out = nullptr;
-  if (cfg->kind != MMR_ENC_MINILM && cfg->kind != MMR_ENC_CLIP_TEXT && cfg->kind != MMR_ENC_CROSS)
-    return fail(MMR_ERR_INVALID, "unknown encoder kind %d", cfg->kind);
+// Device check and allocation of a validated config (cfg: text kinds; vc: also given for MMR_ENC_CLIP_VISION).
+static int encoder_new(int device, const mmr_encoder_config* cfg, const mmr_vision_config* vc, mmr_encoder** out) {
   const int H = cfg->hidden, I = cfg->intermediate;
-  if ((H != 384 && H != 512) || H % cfg->heads != 0 || (H / cfg->heads != 32 && H / cfg->heads != 64))
-    return fail(MMR_ERR_UNSUPPORTED, "hidden %d / heads %d: kernels are built for hidden 384 or 512 with head dim 32 or 64", H, cfg->heads);
-  if (I % 128 != 0 || I % 64 != 0 || (3 * H) % 128 != 0) return fail(MMR_ERR_UNSUPPORTED, "intermediate size must be a multiple of 128");
-  if (cfg->layers < 1 || cfg->vocab_size < 1 || cfg->max_positions < 1) return fail(MMR_ERR_INVALID, "bad config");
   int major = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
   if (major != 10) return fail(MMR_ERR_CUDA, "device %d is not sm_100: the encoders have no other backend", device);
@@ -81,13 +80,18 @@ extern "C" int mmr_encoder_create(int device, const mmr_encoder_config* cfg, mmr
   mmr_encoder* e = new mmr_encoder();
   e->device = device;
   e->cfg = *cfg;
-  e->out_dim = cfg->kind == MMR_ENC_CROSS ? 1 : (cfg->kind == MMR_ENC_CLIP_TEXT ? cfg->proj_dim : H);
+  if (vc) {
+    e->vcfg = *vc;
+    e->patch_cols = vc->channels * vc->patch_size * vc->patch_size;
+  }
+  const bool clip = cfg->kind == MMR_ENC_CLIP_TEXT || cfg->kind == MMR_ENC_CLIP_VISION;
+  e->out_dim = cfg->kind == MMR_ENC_CROSS ? 1 : (clip ? cfg->proj_dim : H);
   e->layers.resize(cfg->layers);
   int rc = MMR_OK;
   auto A = [&](void** p, size_t bytes) { if (rc == MMR_OK) rc = dev_alloc(e, p, bytes); };
-  A((void**)&e->word, size_t(cfg->vocab_size) * H * 4);
+  if (cfg->kind != MMR_ENC_CLIP_VISION) A((void**)&e->word, size_t(cfg->vocab_size) * H * 4);
   A((void**)&e->pos, size_t(cfg->max_positions) * H * 4);
-  if (cfg->kind != MMR_ENC_CLIP_TEXT) {
+  if (!clip) {
     A((void**)&e->type_emb, size_t(std::max(cfg->type_vocab, 1)) * H * 4);
     A((void**)&e->emb_ln_w, H * 4);
     A((void**)&e->emb_ln_b, H * 4);
@@ -95,6 +99,14 @@ extern "C" int mmr_encoder_create(int device, const mmr_encoder_config* cfg, mmr
     A((void**)&e->final_ln_w, H * 4);
     A((void**)&e->final_ln_b, H * 4);
     A((void**)&e->proj_w, size_t(cfg->proj_dim) * H * 4);
+  }
+  if (cfg->kind == MMR_ENC_CLIP_VISION) {
+    A((void**)&e->cls_emb, H * 4);
+    A((void**)&e->pre_ln_w, H * 4);
+    A((void**)&e->pre_ln_b, H * 4);
+    A((void**)&e->patch_w, size_t(H) * e->patch_cols * 2);
+    if (rc == MMR_OK && !make_map(&e->m_patch_w, e->patch_w, H, e->patch_cols, ENC_BM))
+      rc = fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed for the patch embedding weight");
   }
   if (cfg->kind == MMR_ENC_CROSS) {
     A((void**)&e->pool_w, size_t(H) * H * 4);
@@ -127,6 +139,52 @@ extern "C" int mmr_encoder_create(int device, const mmr_encoder_config* cfg, mmr
   return MMR_OK;
 }
 
+extern "C" int mmr_encoder_create(int device, const mmr_encoder_config* cfg, mmr_encoder** out) {
+  if (!out || !cfg) return fail(MMR_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  if (cfg->kind != MMR_ENC_MINILM && cfg->kind != MMR_ENC_CLIP_TEXT && cfg->kind != MMR_ENC_CROSS)
+    return fail(MMR_ERR_INVALID, "unknown encoder kind %d", cfg->kind);
+  const int H = cfg->hidden, I = cfg->intermediate;
+  if ((H != 384 && H != 512) || H % cfg->heads != 0 || (H / cfg->heads != 32 && H / cfg->heads != 64))
+    return fail(MMR_ERR_UNSUPPORTED, "hidden %d / heads %d: kernels are built for hidden 384 or 512 with head dim 32 or 64", H, cfg->heads);
+  if (I % 128 != 0 || I % 64 != 0 || (3 * H) % 128 != 0) return fail(MMR_ERR_UNSUPPORTED, "intermediate size must be a multiple of 128");
+  if (cfg->layers < 1 || cfg->vocab_size < 1 || cfg->max_positions < 1) return fail(MMR_ERR_INVALID, "bad config");
+  return encoder_new(device, cfg, nullptr, out);
+}
+
+extern "C" int mmr_encoder_create_vision(int device, const mmr_vision_config* vc, mmr_encoder** out) {
+  if (!out || !vc) return fail(MMR_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  const int H = vc->hidden;
+  if (H != 768 || vc->heads < 1 || H % vc->heads != 0 || H / vc->heads != 64)
+    return fail(MMR_ERR_UNSUPPORTED, "hidden %d / heads %d: the vision tower is built for hidden 768 with head dim 64", H, vc->heads);
+  if (vc->layers < 1) return fail(MMR_ERR_INVALID, "layers = %d: must be >= 1", vc->layers);
+  if (vc->channels < 1 || vc->patch_size < 1 || vc->image_size < 1)
+    return fail(MMR_ERR_INVALID, "channels %d / image_size %d / patch_size %d: must be >= 1", vc->channels, vc->image_size, vc->patch_size);
+  if (vc->image_size % vc->patch_size != 0)
+    return fail(MMR_ERR_INVALID, "image_size %d is not a multiple of patch_size %d", vc->image_size, vc->patch_size);
+  const int64_t cols = int64_t(vc->channels) * vc->patch_size * vc->patch_size;
+  if (cols % 64 != 0 || cols > (1 << 20))
+    return fail(MMR_ERR_UNSUPPORTED, "channels * patch_size^2 = %lld: the patch GEMM needs a multiple of 64 (at most 2^20)", (long long)cols);
+  if (vc->intermediate < 128 || vc->intermediate % 128 != 0)
+    return fail(MMR_ERR_UNSUPPORTED, "intermediate size %d must be a positive multiple of 128", vc->intermediate);
+  const int64_t grid = vc->image_size / vc->patch_size, tokens = grid * grid + 1;
+  if (tokens > 330)
+    return fail(MMR_ERR_UNSUPPORTED, "%lld tokens per image (%lld patches + class token): the fp32 attention at head dim 64 takes 330 at most",
+                (long long)tokens, (long long)(tokens - 1));
+  if (vc->proj_dim < 1 || vc->proj_dim > H) return fail(MMR_ERR_INVALID, "proj_dim %d: must be in [1, hidden = %d]", vc->proj_dim, H);
+  mmr_encoder_config cfg{};
+  cfg.kind = MMR_ENC_CLIP_VISION;
+  cfg.hidden = H;
+  cfg.layers = vc->layers;
+  cfg.heads = vc->heads;
+  cfg.intermediate = vc->intermediate;
+  cfg.max_positions = int32_t(tokens);
+  cfg.proj_dim = vc->proj_dim;
+  cfg.ln_eps = vc->ln_eps;
+  return encoder_new(device, &cfg, vc, out);
+}
+
 extern "C" int mmr_encoder_destroy(mmr_encoder* e) {
   if (!e) return MMR_OK;
   cudaSetDevice(e->device);
@@ -151,6 +209,10 @@ static bool weight_slot(mmr_encoder* e, const std::string& name, void** dst, int
   if (name == "final_ln_w") return set(e->final_ln_w, H);
   if (name == "final_ln_b") return set(e->final_ln_b, H);
   if (name == "proj_w") return set(e->proj_w, int64_t(e->cfg.proj_dim) * H);
+  if (name == "patch_w") return set(e->patch_w, int64_t(H) * e->patch_cols, true);
+  if (name == "cls_emb") return set(e->cls_emb, H);
+  if (name == "pre_ln_w") return set(e->pre_ln_w, H);
+  if (name == "pre_ln_b") return set(e->pre_ln_b, H);
   if (name == "pooler_w") return set(e->pool_w, int64_t(H) * H);
   if (name == "pooler_b") return set(e->pool_b, H);
   if (name == "cls_w") return set(e->cls_w, H);
@@ -207,7 +269,8 @@ static int ensure_arena(mmr_encoder* e, int tokens, int seqs) {
   CUDA_TRY(cudaMalloc((void**)&e->qkv, size_t(cap) * 3 * H * 4));  e->owned.push_back(e->qkv);
   CUDA_TRY(cudaMalloc((void**)&e->x16, size_t(cap) * H * 2));      e->owned.push_back(e->x16);
   CUDA_TRY(cudaMalloc((void**)&e->ctx16, size_t(cap) * H * 2));    e->owned.push_back(e->ctx16);
-  CUDA_TRY(cudaMalloc((void**)&e->h16, size_t(cap) * I * 2));      e->owned.push_back(e->h16);
+  // h16 also holds a vision pass's patch matrix (B * NP < tokens rows of C * P * P), read before the first FFN1 writes h16
+  CUDA_TRY(cudaMalloc((void**)&e->h16, size_t(cap) * std::max(I, e->patch_cols) * 2)); e->owned.push_back(e->h16);
   CUDA_TRY(cudaMalloc((void**)&e->d_ids, size_t(cap) * 3 * 4));    e->owned.push_back(e->d_ids);
   e->d_mask = e->d_ids + cap;
   e->d_types = e->d_ids + 2 * size_t(cap);
@@ -353,30 +416,130 @@ static int launch_attention(bool tensor_cores, int B, int S, int H, int heads, i
   return MMR_OK;
 }
 
+// Tensor maps of the activation buffers for a pass of M tokens (TMA zero-fills rows past M, so they depend on the live
+// token count); patch_rows > 0 (vision) also maps the patch matrix.  Box rows of an activation map = the token tile of the
+// GEMMs that read it: x16 feeds QKV (N = 3H) and FFN1 (N = I), ctx16 the out-projection and h16 FFN2 (both N = H), the patch
+// matrix the patch GEMM (N = H).
+static int ensure_maps(mmr_encoder* e, int M, int H, int patch_rows) {
+  if (e->maps_tokens == M && e->maps_narrow == options().enc_narrow_tiles) return MMR_OK;
+  const int I = e->cfg.intermediate;
+  e->nt_x = enc_token_tile_for(M, std::min(3 * H, I));
+  e->nt_ctx = enc_token_tile_for(M, H);
+  e->nt_h = enc_token_tile_for(M, H);
+  if (!make_map(&e->m_x16, e->x16, M, H, e->nt_x) || !make_map(&e->m_ctx16, e->ctx16, M, H, e->nt_ctx) ||
+      !make_map(&e->m_h16, e->h16, M, I, e->nt_h))
+    return fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed for the activations");
+  if (patch_rows > 0) {
+    e->nt_patch = enc_token_tile_for(patch_rows, H);
+    if (!make_map(&e->m_patch, e->h16, patch_rows, e->patch_cols, e->nt_patch))
+      return fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed for the patch matrix");
+  }
+  e->maps_tokens = M;
+  e->maps_narrow = options().enc_narrow_tiles;
+  return MMR_OK;
+}
+
+// Attention kernel of a model: the cross-encoder (rerank passages: 128-512 tokens) runs both attention contractions on the
+// tensor cores, whatever the sequence length (kernel choice by model, never by batch shape); MMR_ENC_ATT_MMA=0: fp32 kernel
+// everywhere, =2: every model from ATC_MIN_S tokens on (measurement)
+static bool attention_on_tensor_cores(const mmr_encoder* e, int S) {
+  const int att_opt = options().enc_att_mma;
+  return att_opt == 2 ? S >= ATC_MIN_S : (att_opt == 1 && e->cfg.kind == MMR_ENC_CROSS);
+}
+
+// The pre-LN layer stack of both CLIP towers over the fp32 residual stream e->x [B * S, H]:
+//   h = LN1(x); x = x + out_proj(attention(qkv(h))); h = LN2(x); x = x + fc2(quick_gelu(fc1(h)))
+// Text: causal with the padding mask; vision: neither.  fuse_ln folds LN1 / LN2 into the QKV / FC1 GEMMs (H <= 512 only).
+template <int H>
+static int preln_layers(mmr_encoder* e, int B, int S, bool att_mma, int causal, const int32_t* mask, bool fuse_ln, cudaStream_t st) {
+  const mmr_encoder_config& c = e->cfg;
+  const int M = B * S, I = c.intermediate;
+  const int wpb = 8;
+  const dim3 rows_grid((M + wpb - 1) / wpb), rows_block(wpb * 32);
+  for (LayerW& L : e->layers) {
+    int rc;
+    if (fuse_ln) {
+      rc = launch_gemm_ln<EPI_BIAS_F32>(L.m_qkv, e->m_x16, M, 3 * H, H, L.qkv_b, e->qkv, nullptr, e->x, L.ln1_w, L.ln1_b, c.ln_eps,
+                                        nullptr, st);
+    } else {
+      CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->x, L.ln1_w, L.ln1_b, c.ln_eps, M, (float*)nullptr,
+                          e->x16));
+      mmr_g_launches++;
+      rc = launch_gemm<EPI_BIAS_F32>(L.m_qkv, e->m_x16, e->nt_x, M, 3 * H, H, L.qkv_b, nullptr, e->qkv, nullptr, st);
+    }
+    if (rc != MMR_OK) return rc;
+    rc = launch_attention(att_mma, B, S, H, c.heads, causal, e->qkv, mask, e->ctx16, st);
+    if (rc != MMR_OK) return rc;
+    rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_o, e->m_ctx16, e->nt_ctx, M, H, H, L.o_b, e->x, e->x, nullptr, st);
+    if (rc != MMR_OK) return rc;
+    if (fuse_ln) {
+      rc = launch_gemm_ln<EPI_QUICKGELU_BF16>(L.m_fc1, e->m_x16, M, I, H, L.fc1_b, nullptr, e->h16, e->x, L.ln2_w, L.ln2_b, c.ln_eps,
+                                              nullptr, st);
+    } else {
+      CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->x, L.ln2_w, L.ln2_b, c.ln_eps, M, (float*)nullptr,
+                          e->x16));
+      mmr_g_launches++;
+      rc = launch_gemm<EPI_QUICKGELU_BF16>(L.m_fc1, e->m_x16, e->nt_x, M, I, H, L.fc1_b, nullptr, nullptr, e->h16, st);
+    }
+    if (rc != MMR_OK) return rc;
+    rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_fc2, e->m_h16, e->nt_h, M, H, I, L.fc2_b, e->x, e->x, nullptr, st);
+    if (rc != MMR_OK) return rc;
+  }
+  return MMR_OK;
+}
+
+// The post-LN layer stack of BERT (MiniLM, cross-encoder): x = LN1(x + out_proj(attention(qkv(x))));
+// x = LN2(x + fc2(gelu(fc1(x)))), with the padding mask.  fuse_ln folds LN1 into FC1 and LN2 into the next layer's QKV GEMM.
+template <int H>
+static int postln_layers(mmr_encoder* e, int B, int S, bool att_mma, bool fuse_ln, cudaStream_t st) {
+  const mmr_encoder_config& c = e->cfg;
+  const int M = B * S, I = c.intermediate;
+  const int wpb = 8;
+  const dim3 rows_grid((M + wpb - 1) / wpb), rows_block(wpb * 32);
+  const LayerW* prev = nullptr;   // BERT: the layer whose closing LayerNorm (ln2 over e->tmp) is still pending
+  for (LayerW& L : e->layers) {
+    int rc;
+    if (prev != nullptr) {   // BERT, fused: x = LN2_prev(tmp) computed by this layer's QKV GEMM
+      rc = launch_gemm_ln<EPI_BIAS_F32>(L.m_qkv, e->m_x16, M, 3 * H, H, L.qkv_b, e->qkv, nullptr, e->tmp, prev->ln2_w, prev->ln2_b,
+                                        c.ln_eps, e->x, st);
+    } else {
+      rc = launch_gemm<EPI_BIAS_F32>(L.m_qkv, e->m_x16, e->nt_x, M, 3 * H, H, L.qkv_b, nullptr, e->qkv, nullptr, st);
+    }
+    if (rc != MMR_OK) return rc;
+    rc = launch_attention(att_mma, B, S, H, c.heads, 0, e->qkv, e->d_mask, e->ctx16, st);
+    if (rc != MMR_OK) return rc;
+    rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_o, e->m_ctx16, e->nt_ctx, M, H, H, L.o_b, e->x, e->tmp, nullptr, st);
+    if (rc != MMR_OK) return rc;
+    if (fuse_ln) {
+      rc = launch_gemm_ln<EPI_GELU_BF16>(L.m_fc1, e->m_x16, M, I, H, L.fc1_b, nullptr, e->h16, e->tmp, L.ln1_w, L.ln1_b, c.ln_eps,
+                                         e->x, st);
+    } else {
+      CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->tmp, L.ln1_w, L.ln1_b, c.ln_eps, M, e->x, e->x16));
+      mmr_g_launches++;
+      rc = launch_gemm<EPI_GELU_BF16>(L.m_fc1, e->m_x16, e->nt_x, M, I, H, L.fc1_b, nullptr, nullptr, e->h16, st);
+    }
+    if (rc != MMR_OK) return rc;
+    rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_fc2, e->m_h16, e->nt_h, M, H, I, L.fc2_b, e->x, e->tmp, nullptr, st);
+    if (rc != MMR_OK) return rc;
+    if (fuse_ln && &L != &e->layers.back()) {
+      prev = &L;   // LN2 rides in the next layer's QKV GEMM
+    } else {
+      CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->tmp, L.ln2_w, L.ln2_b, c.ln_eps, M, e->x, e->x16));
+      mmr_g_launches++;
+    }
+  }
+  return MMR_OK;
+}
+
 template <int H>
 static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t st) {
   const mmr_encoder_config& c = e->cfg;
-  const int M = B * S, I = c.intermediate, DH = H / c.heads;
+  const int M = B * S, DH = H / c.heads;
   const bool clip = c.kind == MMR_ENC_CLIP_TEXT;
   const int wpb = 8;
   const dim3 rows_grid((M + wpb - 1) / wpb), rows_block(wpb * 32);
-  if (e->maps_tokens != M || e->maps_narrow != options().enc_narrow_tiles) {   // the activation maps depend on the live token count (TMA zero-fills rows past it)
-    // box rows of an activation map = the token tile of the GEMMs that read it: x16 feeds QKV (N = 3H) and FFN1 (N = I),
-    // ctx16 the out-projection and h16 FFN2 (both N = H)
-    e->nt_x = enc_token_tile_for(M, std::min(3 * H, I));
-    e->nt_ctx = enc_token_tile_for(M, H);
-    e->nt_h = enc_token_tile_for(M, H);
-    if (!make_map(&e->m_x16, e->x16, M, H, e->nt_x) || !make_map(&e->m_ctx16, e->ctx16, M, H, e->nt_ctx) ||
-        !make_map(&e->m_h16, e->h16, M, I, e->nt_h))
-      return fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed for the activations");
-    e->maps_tokens = M;
-    e->maps_narrow = options().enc_narrow_tiles;
-  }
-  // the cross-encoder (rerank passages: 128-512 tokens) runs both attention contractions on the tensor cores, whatever the
-  // sequence length (kernel choice by model, never by batch shape); MMR_ENC_ATT_MMA=0: fp32 kernel everywhere, =2: every model
-  // from ATC_MIN_S tokens on (measurement)
-  const int att_opt = options().enc_att_mma;
-  const bool att_mma = att_opt == 2 ? S >= ATC_MIN_S : (att_opt == 1 && c.kind == MMR_ENC_CROSS);
+  if (const int rc = ensure_maps(e, M, H, 0); rc != MMR_OK) return rc;
+  const bool att_mma = attention_on_tensor_cores(e, S);
   size_t att_smem = 0;
   if (const int rc = attention_smem(att_mma, DH, S, &att_smem); rc != MMR_OK) return rc;   // before the first launch
 
@@ -395,67 +558,8 @@ static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t 
   // costs no more than the LayerNorm it carried, and every CTA of the GEMM repeats its token tile's LayerNorm.
   const int fuse_opt = options().enc_fuse_ln;
   const bool fuse_ln = fuse_opt == 2 ? enc_token_tile(M) == 64 : (fuse_opt == 1 && M <= 16);
-  const LayerW* prev = nullptr;   // BERT: the layer whose closing LayerNorm (ln2 over e->tmp) is still pending
-  for (LayerW& L : e->layers) {
-    int rc;
-    if (clip) {  // pre-LN: h = LN1(x)
-      if (fuse_ln) {
-        rc = launch_gemm_ln<EPI_BIAS_F32>(L.m_qkv, e->m_x16, M, 3 * H, H, L.qkv_b, e->qkv, nullptr, e->x, L.ln1_w, L.ln1_b, c.ln_eps,
-                                          nullptr, st);
-      } else {
-        CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->x, L.ln1_w, L.ln1_b, c.ln_eps, M,
-                            (float*)nullptr, e->x16));
-        mmr_g_launches++;
-        rc = launch_gemm<EPI_BIAS_F32>(L.m_qkv, e->m_x16, e->nt_x, M, 3 * H, H, L.qkv_b, nullptr, e->qkv, nullptr, st);
-      }
-    } else if (prev != nullptr) {   // BERT, fused: x = LN2_prev(tmp) computed by this layer's QKV GEMM
-      rc = launch_gemm_ln<EPI_BIAS_F32>(L.m_qkv, e->m_x16, M, 3 * H, H, L.qkv_b, e->qkv, nullptr, e->tmp, prev->ln2_w, prev->ln2_b,
-                                        c.ln_eps, e->x, st);
-    } else {
-      rc = launch_gemm<EPI_BIAS_F32>(L.m_qkv, e->m_x16, e->nt_x, M, 3 * H, H, L.qkv_b, nullptr, e->qkv, nullptr, st);
-    }
-    if (rc != MMR_OK) return rc;
-    rc = launch_attention(att_mma, B, S, H, c.heads, clip ? 1 : 0, e->qkv, e->d_mask, e->ctx16, st);
-    if (rc != MMR_OK) return rc;
-    if (clip) {
-      // x = x + out_proj(ctx); h = LN2(x); x = x + fc2(quick_gelu(fc1(h)))
-      rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_o, e->m_ctx16, e->nt_ctx, M, H, H, L.o_b, e->x, e->x, nullptr, st);
-      if (rc != MMR_OK) return rc;
-      if (fuse_ln) {
-        rc = launch_gemm_ln<EPI_QUICKGELU_BF16>(L.m_fc1, e->m_x16, M, I, H, L.fc1_b, nullptr, e->h16, e->x, L.ln2_w, L.ln2_b, c.ln_eps,
-                                                nullptr, st);
-      } else {
-        CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->x, L.ln2_w, L.ln2_b, c.ln_eps, M,
-                            (float*)nullptr, e->x16));
-        mmr_g_launches++;
-        rc = launch_gemm<EPI_QUICKGELU_BF16>(L.m_fc1, e->m_x16, e->nt_x, M, I, H, L.fc1_b, nullptr, nullptr, e->h16, st);
-      }
-      if (rc != MMR_OK) return rc;
-      rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_fc2, e->m_h16, e->nt_h, M, H, I, L.fc2_b, e->x, e->x, nullptr, st);
-      if (rc != MMR_OK) return rc;
-    } else {
-      // post-LN (BERT): x = LN1(x + out_proj(ctx)); x = LN2(x + fc2(gelu(fc1(x))))
-      rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_o, e->m_ctx16, e->nt_ctx, M, H, H, L.o_b, e->x, e->tmp, nullptr, st);
-      if (rc != MMR_OK) return rc;
-      if (fuse_ln) {
-        rc = launch_gemm_ln<EPI_GELU_BF16>(L.m_fc1, e->m_x16, M, I, H, L.fc1_b, nullptr, e->h16, e->tmp, L.ln1_w, L.ln1_b, c.ln_eps,
-                                           e->x, st);
-      } else {
-        CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->tmp, L.ln1_w, L.ln1_b, c.ln_eps, M, e->x, e->x16));
-        mmr_g_launches++;
-        rc = launch_gemm<EPI_GELU_BF16>(L.m_fc1, e->m_x16, e->nt_x, M, I, H, L.fc1_b, nullptr, nullptr, e->h16, st);
-      }
-      if (rc != MMR_OK) return rc;
-      rc = launch_gemm<EPI_BIAS_RES_F32>(L.m_fc2, e->m_h16, e->nt_h, M, H, I, L.fc2_b, e->x, e->tmp, nullptr, st);
-      if (rc != MMR_OK) return rc;
-      if (fuse_ln && &L != &e->layers.back()) {
-        prev = &L;   // LN2 rides in the next layer's QKV GEMM
-      } else {
-        CUDA_TRY(launch_pdl(layernorm_kernel<H>, rows_grid, rows_block, 0, st, e->tmp, L.ln2_w, L.ln2_b, c.ln_eps, M, e->x, e->x16));
-        mmr_g_launches++;
-      }
-    }
-  }
+  const int rc = clip ? preln_layers<H>(e, B, S, att_mma, 1, e->d_mask, fuse_ln, st) : postln_layers<H>(e, B, S, att_mma, fuse_ln, st);
+  if (rc != MMR_OK) return rc;
   // head
   if (c.kind == MMR_ENC_MINILM)
     CUDA_TRY(launch_pdl(mean_pool_norm_kernel, dim3(B), dim3(H), 0, st, e->x, e->d_mask, S, H, out_dev));
@@ -469,9 +573,64 @@ static int forward_t(mmr_encoder* e, int B, int S, float* out_dev, cudaStream_t 
   return MMR_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ CLIP vision tower
+constexpr int VIS_H = 768;
+
+// The vision front end for B images of C x S_img x S_img pixels, patch size P: patchify -> patch16 [B * NP, C P P] bf16
+// (tensor map m_patch, token tile nt), patch GEMM (no bias) -> patch_out fp32 [B * NP, H], class token + positions +
+// pre-LayerNorm -> x fp32 [B * (NP + 1), H].  The forward pass and mmr_debug_enc_patch_embed both launch through here.
+static int launch_vision_front(int B, int C, int S_img, int P, const float* pixels, __nv_bfloat16* patch16, const CUtensorMap& m_patch_w,
+                               const CUtensorMap& m_patch, int nt, float* patch_out, const float* cls, const float* pos,
+                               const float* ln_g, const float* ln_b, float eps, float* x, cudaStream_t st) {
+  const int np = (S_img / P) * (S_img / P), T = np + 1, M = B * T;
+  CUDA_TRY(launch_pdl(patchify_kernel, dim3(B * np), dim3(256), 0, st, pixels, C, S_img, P, patch16));
+  mmr_g_launches++;
+  const int rc = launch_gemm<EPI_BIAS_F32>(m_patch_w, m_patch, nt, B * np, VIS_H, C * P * P, nullptr, nullptr, patch_out, nullptr, st);
+  if (rc != MMR_OK) return rc;
+  const int wpb = 8;
+  CUDA_TRY(launch_pdl(vision_embed_kernel<VIS_H>, dim3((M + wpb - 1) / wpb), dim3(wpb * 32), 0, st, patch_out, cls, pos, ln_g, ln_b,
+                      eps, M, T, x));
+  mmr_g_launches++;
+  return MMR_OK;
+}
+
+static int forward_vision(mmr_encoder* e, const float* pixels, int B, float* out_dev, cudaStream_t st) {
+  const mmr_encoder_config& c = e->cfg;
+  const mmr_vision_config& v = e->vcfg;
+  const int T = c.max_positions, M = B * T;
+  if (const int rc = ensure_maps(e, M, VIS_H, B * (T - 1)); rc != MMR_OK) return rc;
+  const bool att_mma = attention_on_tensor_cores(e, T);
+  size_t att_smem = 0;
+  if (const int rc = attention_smem(att_mma, VIS_H / c.heads, T, &att_smem); rc != MMR_OK) return rc;   // before the first launch
+  int rc = launch_vision_front(B, v.channels, v.image_size, v.patch_size, pixels, e->h16, e->m_patch_w, e->m_patch, e->nt_patch, e->tmp,
+                               e->cls_emb, e->pos, e->pre_ln_w, e->pre_ln_b, c.ln_eps, e->x, st);
+  if (rc != MMR_OK) return rc;
+  // no mask, not causal; the LayerNorm-folded GEMM holds K <= 512 and is never used at hidden 768
+  rc = preln_layers<VIS_H>(e, B, T, att_mma, 0, nullptr, false, st);
+  if (rc != MMR_OK) return rc;
+  CUDA_TRY(launch_pdl(clip_head_kernel, dim3(B), dim3(VIS_H), size_t(VIS_H + c.proj_dim) * 4, st, e->x, (const int32_t*)nullptr, T,
+                      VIS_H, 0, e->final_ln_w, e->final_ln_b, c.ln_eps, e->proj_w, c.proj_dim, out_dev));
+  mmr_g_launches++;
+  return MMR_OK;
+}
+
+extern "C" int mmr_encoder_forward_pixels(mmr_encoder* e, const float* pixels_dev, int32_t B, float* out_dev, void* stream) {
+  if (B < 1 || B > 65535) return fail(MMR_ERR_INVALID, "B = %d: must be in [1, 65535]", B);   // 65535: the attention grid's y
+  if (!e || !pixels_dev || !out_dev) return fail(MMR_ERR_INVALID, "NULL argument");
+  if (e->cfg.kind != MMR_ENC_CLIP_VISION)
+    return fail(MMR_ERR_INVALID, "encoder kind %d takes token ids (mmr_encoder_forward), not pixels", e->cfg.kind);
+  std::lock_guard<std::mutex> guard(e->mu);
+  CUDA_TRY(cudaSetDevice(e->device));
+  const int rc = ensure_arena(e, B * e->cfg.max_positions, B);
+  if (rc != MMR_OK) return rc;
+  return forward_vision(e, pixels_dev, B, out_dev, static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int mmr_encoder_forward(mmr_encoder* e, const int32_t* input_ids_host, const int32_t* attention_mask_host,
                                    const int32_t* token_type_host, int32_t B, int32_t S, float* out_dev, void* stream) {
   if (!e || !input_ids_host || !out_dev) return fail(MMR_ERR_INVALID, "NULL argument");
+  if (e->cfg.kind == MMR_ENC_CLIP_VISION)
+    return fail(MMR_ERR_INVALID, "a vision encoder takes pixels (mmr_encoder_forward_pixels), not token ids");
   if (B < 1 || S < 1) return fail(MMR_ERR_INVALID, "B and S must be >= 1");
   if (S > e->cfg.max_positions) return fail(MMR_ERR_INVALID, "sequence length %d > max_positions %d", S, e->cfg.max_positions);
   if (S > 512) return fail(MMR_ERR_UNSUPPORTED, "sequence length %d > 512", S);
@@ -589,4 +748,28 @@ extern "C" int mmr_debug_enc_layernorm(int32_t H, int32_t M, const float* x_dev,
     CUDA_TRY(launch_pdl(layernorm_kernel<512>, grid, block, 0, st, x_dev, g_dev, b_dev, eps, M, out_f32_dev, o16));
   mmr_g_launches++;
   return MMR_OK;
+}
+
+extern "C" int mmr_debug_enc_patch_embed(int32_t H, int32_t C, int32_t image_size, int32_t patch, int32_t B, const float* pixels_dev,
+                                         const void* patch_w_dev, const float* cls_dev, const float* pos_dev, const float* ln_g_dev,
+                                         const float* ln_b_dev, float ln_eps, void* patch16_dev, float* patch_out_dev, float* x_dev,
+                                         void* stream) {
+  if (H != VIS_H) return fail(MMR_ERR_INVALID, "H = %d: the vision front end is built for hidden 768", H);
+  if (C < 1 || patch < 1 || image_size < 1)
+    return fail(MMR_ERR_INVALID, "C = %d, image_size = %d, patch = %d: must be >= 1", C, image_size, patch);
+  if (image_size % patch != 0) return fail(MMR_ERR_INVALID, "image_size %d is not a multiple of patch %d", image_size, patch);
+  const int64_t cols = int64_t(C) * patch * patch, grid = image_size / patch;
+  if (cols % 64 != 0 || cols > (1 << 20)) return fail(MMR_ERR_INVALID, "C * patch^2 = %lld: must be a multiple of 64 (at most 2^20)", (long long)cols);
+  if (B < 1 || B > 65535) return fail(MMR_ERR_INVALID, "B = %d: must be in [1, 65535]", B);
+  if (int64_t(B) * (grid * grid + 1) > (1 << 22)) return fail(MMR_ERR_INVALID, "B x tokens per image must be <= 2^22");
+  if (!pixels_dev || !cls_dev || !pos_dev || !ln_g_dev || !ln_b_dev || !patch_out_dev || !x_dev) return fail(MMR_ERR_INVALID, "NULL argument");
+  if (!patch_w_dev || !patch16_dev || !aligned16(patch_w_dev) || !aligned16(patch16_dev))
+    return fail(MMR_ERR_INVALID, "patch_w and patch16 must be 16-byte aligned device pointers");
+  const int rows = B * int(grid * grid);
+  const int nt = enc_token_tile_for(rows, H);   // the forward pass's tile for this patch count
+  CUtensorMap mw, mx;
+  if (!make_map(&mw, patch_w_dev, H, int(cols), ENC_BM) || !make_map(&mx, patch16_dev, rows, int(cols), nt))
+    return fail(MMR_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+  return launch_vision_front(B, C, image_size, patch, pixels_dev, static_cast<__nv_bfloat16*>(patch16_dev), mw, mx, nt, patch_out_dev,
+                             cls_dev, pos_dev, ln_g_dev, ln_b_dev, ln_eps, x_dev, static_cast<cudaStream_t>(stream));
 }

@@ -10,9 +10,14 @@ device tensor that `ResidentIndex.search` consumes directly:
     CLIP ViT-B/32 text tower (openai/clip-vit-base-patch32)   -> ImageQueryEncoder  == embed_query_for_images
     ms-marco-MiniLM-L-6-v2 cross-encoder                      -> DeviceCrossEncoder == CrossEncoder.predict
 
-Weights come from the Hugging Face modules the reference loads (`from_hf_bert` / `from_hf_clip` read their
-state_dict); tokenisation stays on the host (any HF-style callable).  There is no torch / CPU fallback: without the
-library or an sm_100 device construction raises.
+and the model of the ingest side, whose output fills the image rows the scan searches:
+
+    CLIP ViT-B/32 vision tower                                -> ImageEncoder       == embed_images_batch
+
+Weights come from the Hugging Face modules the reference loads (`from_hf_bert` / `from_hf_clip` /
+`from_hf_clip_vision` read their state_dict); tokenisation and image preprocessing stay on the host (any HF-style
+tokenizer, HF's CLIPImageProcessor).  There is no torch / CPU fallback: without the library or an sm_100 device
+construction raises.
 """
 from __future__ import annotations
 
@@ -80,6 +85,36 @@ def hf_clip_text_weights(model) -> Dict[str, torch.Tensor]:
     return out
 
 
+def hf_clip_vision_weights(model) -> Dict[str, torch.Tensor]:
+    """state_dict of a HF CLIPModel / CLIPVisionModelWithProjection -> the C ABI's weight names (vision tower only).
+    The patch embedding's Conv2d weight [H, C, P, P] becomes the GEMM weight [H, C * P * P] ((c, kh, kw) column order)."""
+    sd = model.state_dict()
+    v = "vision_model."
+    pw = sd[v + "embeddings.patch_embedding.weight"]
+    out = {
+        "patch_w": pw.reshape(pw.shape[0], -1),
+        "cls_emb": sd[v + "embeddings.class_embedding"],
+        "pos_emb": sd[v + "embeddings.position_embedding.weight"],
+        "pre_ln_w": sd[v + "pre_layrnorm.weight"],
+        "pre_ln_b": sd[v + "pre_layrnorm.bias"],
+        "final_ln_w": sd[v + "post_layernorm.weight"],
+        "final_ln_b": sd[v + "post_layernorm.bias"],
+        "proj_w": sd["visual_projection.weight"],
+    }
+    i = 0
+    while f"{v}encoder.layers.{i}.self_attn.q_proj.weight" in sd:
+        p = f"{v}encoder.layers.{i}."
+        out[f"L{i}.qkv_w"] = torch.cat([sd[p + f"self_attn.{n}_proj.weight"] for n in ("q", "k", "v")], dim=0)
+        out[f"L{i}.qkv_b"] = torch.cat([sd[p + f"self_attn.{n}_proj.bias"] for n in ("q", "k", "v")], dim=0)
+        out[f"L{i}.o_w"], out[f"L{i}.o_b"] = sd[p + "self_attn.out_proj.weight"], sd[p + "self_attn.out_proj.bias"]
+        out[f"L{i}.ln1_w"], out[f"L{i}.ln1_b"] = sd[p + "layer_norm1.weight"], sd[p + "layer_norm1.bias"]
+        out[f"L{i}.fc1_w"], out[f"L{i}.fc1_b"] = sd[p + "mlp.fc1.weight"], sd[p + "mlp.fc1.bias"]
+        out[f"L{i}.fc2_w"], out[f"L{i}.fc2_b"] = sd[p + "mlp.fc2.weight"], sd[p + "mlp.fc2.bias"]
+        out[f"L{i}.ln2_w"], out[f"L{i}.ln2_b"] = sd[p + "layer_norm2.weight"], sd[p + "layer_norm2.bias"]
+        i += 1
+    return out
+
+
 def _check_supported(cfg, acts) -> None:
     """The kernels implement erf-GELU (BERT), quick-GELU (CLIP) and absolute position embeddings only: any other model
     would run with the wrong math and no error."""
@@ -92,20 +127,25 @@ def _check_supported(cfg, acts) -> None:
 
 
 class DeviceEncoder:
-    """One transformer (MiniLM / CLIP text / cross-encoder) resident on a B200, driven through mmr_encoder_*."""
+    """One transformer (MiniLM / CLIP text / cross-encoder / CLIP vision) resident on a B200, driven through mmr_encoder_*.
+    The vision tower is built with `DeviceEncoder.vision(...)` or `from_hf_clip_vision` and run with `forward_pixels`."""
 
-    def __init__(self, kind: str, *, vocab_size: int, hidden: int, layers: int, heads: int, intermediate: int,
-                 max_positions: int, type_vocab: int = 2, proj_dim: int = 0, eos_token_id: int = 0, ln_eps: float = 1e-12,
-                 device: Any = "cuda:0") -> None:
+    def __init__(self, kind: str, *, vocab_size: int = 0, hidden: int, layers: int, heads: int, intermediate: int,
+                 max_positions: int = 0, type_vocab: int = 2, proj_dim: int = 0, eos_token_id: int = 0, ln_eps: float = 1e-12,
+                 image_size: int = 0, patch_size: int = 0, channels: int = 3, device: Any = "cuda:0") -> None:
         lib = N.lib()
         if not torch.cuda.is_available():
             raise N.NativeError("no CUDA device: the device encoders have no CPU fallback")
         self.kind = kind
         self.device = torch.device(device)
-        self.cfg = N.EncoderConfig(KINDS[kind], vocab_size, hidden, layers, heads, intermediate, max_positions, type_vocab,
-                                   proj_dim, eos_token_id, ln_eps)
         self._handle = C.c_void_p()
-        N.check(lib.mmr_encoder_create(self.device.index or 0, C.byref(self.cfg), C.byref(self._handle)))
+        if kind == "clip_vision":
+            self.cfg = N.VisionConfig(hidden, layers, heads, intermediate, image_size, patch_size, channels, proj_dim, ln_eps)
+            N.check(lib.mmr_encoder_create_vision(self.device.index or 0, C.byref(self.cfg), C.byref(self._handle)))
+        else:
+            self.cfg = N.EncoderConfig(KINDS[kind], vocab_size, hidden, layers, heads, intermediate, max_positions, type_vocab,
+                                       proj_dim, eos_token_id, ln_eps)
+            N.check(lib.mmr_encoder_create(self.device.index or 0, C.byref(self.cfg), C.byref(self._handle)))
         self.out_dim = int(lib.mmr_encoder_out_dim(self._handle))
         self._loaded: List[str] = []
 
@@ -135,6 +175,18 @@ class DeviceEncoder:
         enc.load(weights)
         return enc
 
+    @classmethod
+    def from_hf_clip_vision(cls, model, device: Any = "cuda:0") -> "DeviceEncoder":
+        """CLIP vision tower of a HF CLIPModel or CLIPVisionModelWithProjection (the model `embed_images_batch` runs)."""
+        cfg = getattr(model.config, "vision_config", model.config)
+        _check_supported(cfg, {"quick_gelu"})
+        weights = hf_clip_vision_weights(model)
+        enc = cls("clip_vision", hidden=cfg.hidden_size, layers=cfg.num_hidden_layers, heads=cfg.num_attention_heads,
+                  intermediate=cfg.intermediate_size, proj_dim=int(weights["proj_w"].shape[0]), ln_eps=cfg.layer_norm_eps,
+                  image_size=cfg.image_size, patch_size=cfg.patch_size, channels=cfg.num_channels, device=device)
+        enc.load(weights)
+        return enc
+
     def load(self, weights: Dict[str, torch.Tensor]) -> None:
         lib = N.lib()
         with torch.cuda.device(self.device):
@@ -161,6 +213,23 @@ class DeviceEncoder:
             N.check(N.lib().mmr_encoder_forward(self._handle, ids.ctypes.data, None if mask is None else mask.ctypes.data,
                                                 None if types is None else types.ctypes.data, b, s, out.data_ptr(),
                                                 torch.cuda.current_stream(self.device).cuda_stream))
+        return out
+
+    def forward_pixels(self, pixel_values: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Pixel values [B, C, S, S] (what CLIPImageProcessor returns; any device / dtype) -> [B, proj] fp32 unit-norm image
+        embeddings on the device."""
+        if self.kind != "clip_vision":
+            raise ValueError(f"forward_pixels needs a CLIP vision encoder, not {self.kind!r}")
+        c = self.cfg
+        px = torch.as_tensor(pixel_values).to(device=self.device, dtype=torch.float32).contiguous()
+        if px.dim() != 4 or tuple(px.shape[1:]) != (c.channels, c.image_size, c.image_size):
+            raise ValueError(f"pixel_values must be [B, {c.channels}, {c.image_size}, {c.image_size}], got {tuple(px.shape)}")
+        b = px.shape[0]
+        if out is None:
+            out = torch.empty((b, self.out_dim), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            N.check(N.lib().mmr_encoder_forward_pixels(self._handle, px.data_ptr(), b, out.data_ptr(),
+                                                       torch.cuda.current_stream(self.device).cuda_stream))
         return out
 
     def close(self) -> None:
@@ -235,5 +304,25 @@ class DeviceCrossEncoder:
         return self.predict_device(pairs).cpu().numpy()
 
 
-__all__ = ["DeviceEncoder", "TextQueryEncoder", "ImageQueryEncoder", "DeviceCrossEncoder", "hf_bert_weights",
-           "hf_clip_text_weights"]
+class ImageEncoder:
+    """`embed_images_batch` (app/ml/embeddings.py:73-91) with the CLIP vision tower on the device: images -> unit-norm f32
+    [n, proj].  `processor` is the caller's HF CLIPImageProcessor (resize, centre crop, normalise stay on the host, as
+    tokenisation does for the text encoders); any callable returning {"pixel_values": [n, C, S, S]} works."""
+
+    def __init__(self, processor: Callable, encoder: DeviceEncoder) -> None:
+        self.processor, self.encoder = processor, encoder
+
+    def encode_device(self, images: Sequence[Any]) -> torch.Tensor:
+        px = self.processor(images=list(images), return_tensors="pt")["pixel_values"]
+        return self.encoder.forward_pixels(px)
+
+    def __call__(self, images: Sequence[Any], batch_size: int = 32) -> np.ndarray:
+        images = list(images)
+        if not images:
+            return np.empty((0, self.encoder.out_dim), dtype=np.float32)
+        parts = [self.encode_device(images[i:i + batch_size]).cpu().numpy() for i in range(0, len(images), batch_size)]
+        return np.concatenate(parts, axis=0)
+
+
+__all__ = ["DeviceEncoder", "TextQueryEncoder", "ImageQueryEncoder", "ImageEncoder", "DeviceCrossEncoder", "hf_bert_weights",
+           "hf_clip_text_weights", "hf_clip_vision_weights"]
