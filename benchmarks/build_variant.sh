@@ -4,7 +4,7 @@ set -e
 NAME=$1; shift
 P=$(dirname "$0")/../multimodal-rag-for-image-text-search_b200
 mkdir -p $P/build/v_$NAME
-F="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -DMMR_WITH_UMMA"
+F="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC"
 nvcc $F "$@" -c -o $P/build/v_$NAME/mmr_b200.o $P/csrc/mmr_b200.cu &
 nvcc $F "$@" -c -o $P/build/v_$NAME/mmr_encoder.o $P/csrc/mmr_encoder.cu &
 wait

@@ -28,13 +28,10 @@ def main():
         ix.search_ranges(q, 10, [[(0, 50), (200, 900)], [(10, 20)], [], [(0, 6000)]])
         ix.close()
     ix = pkg.ResidentIndex.from_f32(rows, dtype="bf16")
-    for mode, pair in (("ss", "0"), ("ts", "0"), ("ts", "1")):
-        pkg._native.set_option("MMR_UMMA_MODE", mode)
-        pkg._native.set_option("MMR_UMMA_PAIR", pair)
-        for b in (5, 130):
-            q = torch.from_numpy(util.queries(b, 512)).cuda()
-            s, r = ix.search(q, 10)
-            ix.debug_umma_scores(q, 0, 6000)
+    for b in (5, 130):                             # K2: one query tile (single CTAs), two (CTA pairs)
+        q = torch.from_numpy(util.queries(b, 512)).cuda()
+        s, r = ix.search(q, 10)
+        ix.debug_umma_scores(q, 0, 6000)
     parts_s = torch.stack([s, s]); parts_r = torch.stack([r, r + 100000])
     pkg.merge_topk(parts_s, parts_r)
     pkg.fuse((s, r), (s[:, :5].contiguous(), r[:, :5].contiguous()), 4, 0.25)

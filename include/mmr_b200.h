@@ -62,9 +62,8 @@ typedef struct mmr_index mmr_index;
 /* Library / error plumbing. */
 int mmr_abi_version(void);
 const char* mmr_last_error(void);
-/* Switches (DESIGN.md 6a: MMR_PDL, MMR_UMMA_MODE, MMR_UMMA_PAIR, MMR_UMMA_NOPROBE, MMR_UMMA_STAGES, MMR_UMMA_FUSED_PROBE,
- * MMR_FORCE_FAMILY, MMR_UMMA_LOCKSTEP, MMR_UMMA_SKIP_EPI, MMR_INLINE_QUERY, MMR_MAILBOX, MMR_ENC_FUSE_LN, MMR_ENC_ATT_MMA,
- * MMR_ENC_GEMM_SMEM_KB, MMR_ENC_NARROW_TILES; all but MMR_PDL are measurement switches whose defaults are the shipped path).  The
+/* Switches (DESIGN.md 6a: MMR_PDL, MMR_INLINE_QUERY, MMR_MAILBOX, MMR_ENC_FUSE_LN, MMR_ENC_ATT_MMA, MMR_ENC_GEMM_SMEM_KB,
+ * MMR_ENC_NARROW_TILES; all but MMR_PDL are measurement switches whose defaults are the shipped path).  The
  * environment is read once when the library is loaded; these change / read a switch afterwards (value NULL or "" =
  * default).  mmr_get_option returns -1 for an unknown name. */
 int mmr_set_option(const char* name, const char* value);

@@ -114,7 +114,7 @@ def check(status: int) -> None:
 
 
 def set_option(name: str, value) -> None:
-    """Change a library switch (MMR_PDL, MMR_UMMA_MODE, ...) after load; None restores the default."""
+    """Change a library switch (MMR_PDL, MMR_ENC_ATT_MMA, ...) after load; None restores the default."""
     check(lib().mmr_set_option(name.encode(), None if value is None else str(value).encode()))
 
 

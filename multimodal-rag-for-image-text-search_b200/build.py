@@ -43,10 +43,9 @@ def build(force: bool = False, verbose: bool = False, extra: List[str] | None = 
 
     if not force and not needs_build():
         return LIB
-    defines = ["-DMMR_WITH_UMMA"] if os.path.exists(os.path.join(CSRC, "scan_umma.cuh")) else []
     objdir = os.path.join(HERE, "build")
     os.makedirs(objdir, exist_ok=True)
-    common = [_nvcc(), *ARCH_FLAGS, "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", *defines, *(extra or [])]
+    common = [_nvcc(), *ARCH_FLAGS, "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", *(extra or [])]
 
     def compile_one(src: str) -> str:
         obj = os.path.join(objdir, os.path.splitext(src)[0] + ".o")

@@ -47,18 +47,6 @@ __host__ __device__ __forceinline__ uint32_t key_row(uint64_t key) { return 0xFF
 // ------------------------------------------------------------------------------------------------
 struct Options {
   int pdl = 0;            // MMR_PDL=1        pipelined launches (programmatic dependent launch) for K1 / merge_wait
-  int umma_mode = 0;      // MMR_UMMA_MODE    0 = by batch size, 1 = ss, 2 = ts
-  int umma_pair = 1;      // MMR_UMMA_PAIR=0  single CTAs instead of CTA pairs
-  int umma_noprobe = 0;   // MMR_UMMA_NOPROBE=1
-  int umma_stages = 0;    // MMR_UMMA_STAGES=n   cap the single-CTA kernel's index ring at n 16 KB stages (measurement; 0 = as many as fit)
-  int force_family = 0;   // MMR_FORCE_FAMILY 1 = K1, 2 = K2 regardless of batch size
-  int umma_lockstep = 0;      // MMR_UMMA_LOCKSTEP=1  CTA pairs of one row slot keep within a window of tiles (measured SLOWER:
-                              //                      profiles/r02_k2_summary.md; kept as a measurement switch)
-  int umma_fused_probe = 0;  // MMR_UMMA_FUSED_PROBE=1  K2 single-CTA kernel: probe phase + grid barrier + floor inside the scan launch
-                             //                         instead of separate probe / floor launches (measured 22 us SLOWER at 1M rows:
-                             //                         profiles/r02_k2_summary.md; kept as a measurement switch)
-  int umma_skip_epi = 0;  // MMR_UMMA_SKIP_EPI=1  K2 pair mode skips the accumulator read-back (WRONG results; measures what the
-                          //                      MMA pipeline alone reaches: profiles/r02_k2_summary.md)
   int enc_fuse_ln = 0;    // MMR_ENC_FUSE_LN     device encoders: LayerNorm folded into the GEMM behind it (gemm_wt_kernel<.., true>):
                           //                     0 = never (default: measured no faster, profiles/r02_encoder_summary.md), 1 = for
                           //                     passes of <= 16 tokens, 2 = whenever the token tile is 64

@@ -22,9 +22,7 @@
 #include "aux_kernels.cuh"
 #include "common.cuh"
 #include "scan_stream.cuh"
-#ifdef MMR_WITH_UMMA
 #include "scan_umma2.cuh"
-#endif
 
 using namespace mmr;
 
@@ -73,10 +71,8 @@ struct mmr_index {
   void* d_ws = nullptr;
   size_t ws_bytes = 0;
   int cap_b = 0, cap_k = 0;
-#ifdef MMR_WITH_UMMA
   mutable UmmaIndexState umma;
   mutable Umma2IndexState umma2;
-#endif
 };
 
 static int elem_bytes(int dtype) { return dtype == MMR_F32 ? 4 : 2; }
@@ -99,14 +95,6 @@ static int* option_slot(const char* name) {
   Options& o = options();
   if (!name) return nullptr;
   if (!strcmp(name, "MMR_PDL")) return &o.pdl;
-  if (!strcmp(name, "MMR_UMMA_MODE")) return &o.umma_mode;
-  if (!strcmp(name, "MMR_UMMA_PAIR")) return &o.umma_pair;
-  if (!strcmp(name, "MMR_UMMA_NOPROBE")) return &o.umma_noprobe;
-  if (!strcmp(name, "MMR_FORCE_FAMILY")) return &o.force_family;
-  if (!strcmp(name, "MMR_UMMA_LOCKSTEP")) return &o.umma_lockstep;
-  if (!strcmp(name, "MMR_UMMA_SKIP_EPI")) return &o.umma_skip_epi;
-  if (!strcmp(name, "MMR_UMMA_FUSED_PROBE")) return &o.umma_fused_probe;
-  if (!strcmp(name, "MMR_UMMA_STAGES")) return &o.umma_stages;
   if (!strcmp(name, "MMR_ENC_FUSE_LN")) return &o.enc_fuse_ln;
   if (!strcmp(name, "MMR_ENC_ATT_MMA")) return &o.enc_att_mma;
   if (!strcmp(name, "MMR_ENC_GEMM_SMEM_KB")) return &o.enc_gemm_smem_kb;
@@ -115,19 +103,18 @@ static int* option_slot(const char* name) {
   if (!strcmp(name, "MMR_MAILBOX")) return &o.mailbox;
   return nullptr;
 }
-static int parse_option(const char* name, const char* v, int dflt) {
+static int parse_option(const char* v, int dflt) {
   if (!v || !v[0]) return dflt;
-  if (!strcmp(name, "MMR_UMMA_MODE")) return v[0] == 's' ? 1 : (v[0] == 't' ? 2 : 0);
   return atoi(v);
 }
-static const char* kOptionNames[] = {"MMR_PDL", "MMR_UMMA_MODE", "MMR_UMMA_PAIR", "MMR_UMMA_NOPROBE", "MMR_FORCE_FAMILY",
-                                     "MMR_UMMA_LOCKSTEP", "MMR_INLINE_QUERY", "MMR_MAILBOX", "MMR_UMMA_SKIP_EPI", "MMR_UMMA_FUSED_PROBE", "MMR_ENC_FUSE_LN", "MMR_ENC_ATT_MMA", "MMR_ENC_GEMM_SMEM_KB", "MMR_UMMA_STAGES", "MMR_ENC_NARROW_TILES"};
+static const char* kOptionNames[] = {"MMR_PDL", "MMR_INLINE_QUERY", "MMR_MAILBOX", "MMR_ENC_FUSE_LN", "MMR_ENC_ATT_MMA",
+                                     "MMR_ENC_GEMM_SMEM_KB", "MMR_ENC_NARROW_TILES"};
 namespace {
 struct OptionsFromEnv {  // the environment is read once, when the library is loaded
   OptionsFromEnv() {
     for (const char* name : kOptionNames) {
       int* slot = option_slot(name);
-      *slot = parse_option(name, getenv(name), *slot);
+      *slot = parse_option(getenv(name), *slot);
     }
   }
 } g_options_from_env;
@@ -139,7 +126,7 @@ extern "C" int mmr_set_option(const char* name, const char* value) {
   Options defaults;
   Options& o = options();
   const int dflt = *(reinterpret_cast<int*>(&defaults) + (slot - reinterpret_cast<int*>(&o)));
-  *slot = parse_option(name, value, dflt);
+  *slot = parse_option(value, dflt);
   return MMR_OK;
 }
 extern "C" int mmr_get_option(const char* name) {
@@ -200,10 +187,8 @@ extern "C" int mmr_index_update(mmr_index* ix, int64_t n_rows, const void* rows_
   if ((reinterpret_cast<uintptr_t>(rows_dev) & 15) != 0) return fail(MMR_ERR_INVALID, "rows_dev must be 16-byte aligned");
   ix->n_rows = n_rows;
   ix->rows = rows_dev;
-#ifdef MMR_WITH_UMMA
   ix->umma.valid = false;
   ix->umma2.valid = false;
-#endif
   return set_segments(ix, seg, nseg);
 }
 
@@ -457,11 +442,7 @@ static size_t rescore_extra_bytes(int B) {
          align_up(size_t(B), 256);
 }
 static size_t k2_slice_bytes(const mmr_index* ix, int B) {
-#ifdef MMR_WITH_UMMA
   return umma_workspace_bytes(ix->sm_count, ix->dim, B, MMR_MAX_K) + rescore_extra_bytes(B);
-#else
-  return 0;
-#endif
 }
 
 static size_t workspace_bytes_for(const mmr_index* ix, int32_t B, int32_t k, int64_t n_ranges) {
@@ -685,7 +666,6 @@ static int search_varlen_stream(const mmr_index* ix, const float* q, const std::
   return MMR_OK;
 }
 
-#ifdef MMR_WITH_UMMA
 template <typename E, int D>
 static void launch_rescore_ed(const mmr_index* ix, const float* q, const float* cs, const int64_t* cr, const float* qerr, int B,
                               int kc, int k, float* out_s, int64_t* out_r, uint8_t* flags, cudaStream_t st) {
@@ -739,13 +719,11 @@ static int search_rescored(const mmr_index* ix, const float* q, int B, int k, ui
   g_rescore_reruns += reruns;
   return MMR_OK;
 }
-#endif
 
 // One shared row range for the whole batch: K2 when allowed and preferred, else K1 passes.
 static int search_uniform(const mmr_index* ix, QuerySrc q, int B, int k, uint32_t r0, uint32_t r1, float* out_s,
                           int64_t* out_r, uint8_t* ws, size_t ws_total, cudaStream_t st, const ExchangeInfo* xi = nullptr,
                           Completion* done = nullptr) {
-#ifdef MMR_WITH_UMMA
   if (q.dev != nullptr && ix->query_precision != MMR_QP_F32 &&
       umma_preferred(ix->dtype, ix->dim, B, k, int64_t(r1) - r0)) {
     if (ix->query_precision == MMR_QP_RESCORE)
@@ -758,17 +736,12 @@ static int search_uniform(const mmr_index* ix, QuerySrc q, int B, int k, uint32_
     }
     return rc;
   }
-#endif
   return search_uniform_stream(ix, q, B, k, r0, r1, out_s, out_r, ws, st, xi, done);
 }
 
 // true when a uniform batch of B queries would run on the tensor-core family
 static bool uniform_takes_k2(const mmr_index* ix, int B, int k, int64_t nrows) {
-#ifdef MMR_WITH_UMMA
   return ix->query_precision != MMR_QP_F32 && umma_preferred(ix->dtype, ix->dim, B, k, nrows);
-#else
-  return false;
-#endif
 }
 
 static int check_search_args(const mmr_index* ix, int32_t B, int32_t k) {
@@ -1399,7 +1372,6 @@ extern "C" int mmr_multi_search_host(mmr_multi* m, const float* queries_host, in
   return MMR_OK;
 }
 
-#ifdef MMR_WITH_UMMA
 // Debug / validation hook: raw K2 scores (tensor-core contraction only, no top-k) for rows [row_begin, row_end).
 extern "C" int mmr_debug_umma_scores(const mmr_index* ix, const float* queries_dev, int32_t B, int64_t row_begin,
                                      int64_t row_end, float* out_scores_dev, int64_t out_ld, void* workspace_dev,
@@ -1415,12 +1387,6 @@ extern "C" int mmr_debug_umma_scores(const mmr_index* ix, const float* queries_d
   if (rc == MMR_OK) g_launches += umma_launches_per_search();
   return rc;
 }
-#else
-extern "C" int mmr_debug_umma_scores(const mmr_index*, const float*, int32_t, int64_t, int64_t, float*, int64_t, void*,
-                                     size_t, void*) {
-  return fail(MMR_ERR_UNSUPPORTED, "built without the tcgen05 kernel");
-}
-#endif
 
 // ------------------------------------------------------------------------------------------------ K4 / K5
 extern "C" int mmr_merge_topk_strided(const float* scores_dev, const int64_t* rows_dev, int64_t score_shard_stride,

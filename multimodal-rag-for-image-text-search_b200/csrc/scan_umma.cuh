@@ -16,8 +16,8 @@
 //                        one compare against the thread's k-th best score; the rare winner is inserted into the
 //                        thread's private sorted list (shared memory).  No cross-thread traffic.
 // Four accumulators let the MMAs of tile t+1..t+3 run under the epilogue of tile t.
-// CTA (qt, rs) handles query tile qt and row tiles rs, rs + RS, ...; CTAs with equal rs run the same row tiles
-// at the same time, so for B > 128 the index is read from HBM once and from L2 by the other query tiles.
+// CTA (qt, rs) handles query tile qt and row tiles rs, rs + RS, ...  This kernel serves batches of one query tile
+// (B <= 128); larger batches run on CTA pairs (scan_umma2.cuh), which share the same epilogue (k2_epilogue).
 // Per-CTA lists go to global memory; merge_partials_kernel reduces them per query.
 #pragma once
 #include <cuda.h>
@@ -47,25 +47,13 @@ struct UmmaParams {
   uint32_t row_begin, row_end;
   int32_t n_qtiles, n_rslots;
   uint64_t* partial;  // [n_qtiles * n_rslots][128][k]
-  const void* qbf16;  // TS mode: normalised bf16 queries of this launch, [B][D]
+  const void* qbf16;  // pair kernel: normalised bf16 queries of this launch, [B][D]
   const float* floor; // per query: a proven lower bound of its final k-th best score (nullptr = none)
   float* probe_out;   // probe pass: [n_qtiles * n_rslots][128] best score seen by each CTA (nullptr = real scan)
   int32_t probe_tiles;  // probe pass: row tiles per CTA
   uint32_t idesc;       // tcgen05 instruction descriptor (bf16 or fp16 operands)
   float* dump;        // DUMP mode: raw scores [B][dump_ld]
   int64_t dump_ld;
-  // Lockstep window (pair mode, >= 2 query pairs per row slot): progress[rs * n_qpairs + qpair] = tiles started by that
-  // pair; a pair that runs more than `window` tiles ahead of the slowest pair of its row slot waits.  Keeps the pairs that
-  // read the same index tiles within an L2-resident window, so each tile is fetched from HBM once (it was 1.5-2x).
-  uint32_t* progress;
-  int32_t window;
-  int32_t skip_epi;   // measurement only: epilogue hands accumulators back without reading them
-  // Fused probe (single-CTA kernel): the first `fused_probe_tiles` tiles of every CTA are scanned twice -- once keeping only
-  // each query's best score, then, after a grid-wide barrier on `grid_barrier` (zeroed by prep_queries_kernel) and the k-th
-  // largest of the per-CTA bests as a proven floor, for real.  Replaces the separate probe and floor launches.
-  int32_t fused_probe_tiles;
-  float* probe_scratch;     // [n_qtiles * n_rslots][128]
-  uint32_t* grid_barrier;
 };
 
 #ifdef __CUDACC__
@@ -171,16 +159,6 @@ static __device__ __noinline__ uint64_t k2_list_insert(uint64_t* mine, uint32_t*
   return mv;
 }
 
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      :
-      : "r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 __device__ __forceinline__ void tmem_st_x32(uint32_t taddr, const uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
@@ -194,17 +172,118 @@ __device__ __forceinline__ void tmem_st_x32(uint32_t taddr, const uint32_t (&v)[
       : "memory");
 }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint64_t globaltimer_ns_k2() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
+
+// The epilogue warps of both K2 kernels (warps 2-5, thread = query of tile qt): read each accumulator back from tensor
+// memory 32 columns at a time, filter, insert into the thread's candidate list, hand the accumulator back with
+// release(acc); at the end write the list (or, in the probe pass, the best score) out.  acc_tmem = tensor-memory address
+// of accumulator 0; accumulators are NACC x K2_NT columns from there.
+template <bool DUMP, int NACC, typename Release>
+__device__ __forceinline__ void k2_epilogue(const UmmaParams& p, int qt, int rs, int ntiles, uint64_t* lists,
+                                            uint32_t* metas, uint32_t acc_tmem, uint32_t bar_tfull, Release release) {
+  const int warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const int k = p.k;
+  const int quarter = warp & 3;              // TMEM lane quarter this warp may access
+  const int ql = quarter * 32 + lane;        // query within the tile
+  const int qglob = qt * K2_BM + ql;         // query within this launch
+  const bool live = qglob < p.B;
+  const bool warp_live = qt * K2_BM + quarter * 32 < p.B;   // any live query in this warp
+  uint64_t* mine = lists + ql;               // my candidate list: mine[j * 128], j = 0 .. k-1 (unsorted)
+  uint32_t* meta = metas + ql;
+  for (int j = 0; j < k; ++j) mine[size_t(j) * K2_BM] = 0ull;
+  *meta = 0u;
+  // Rows reach a thread in ascending order, so an equal score can never displace a held one: the strict
+  // compare `m > thr_f` is exact.  Padding queries never pass.
+  // A proven lower bound of the final k-th score (from the probe pass) pre-loads the filter, so the scan does
+  // not pay the warm-up in which every row beats an empty list.  `s >= floor` must pass: use the float just below.
+  float thr_floor = -INFINITY;
+  if (p.floor != nullptr && live) {
+    const float f = p.floor[qglob];
+    // the float just below f in the total order; below +-0 that is the largest negative subnormal, not -0.0
+    // (which compares equal to 0 and would reject every row scoring exactly 0, e.g. for an all-zero query)
+    if (f > -INFINITY) {
+      const uint32_t o = f32_orderable(f);
+      thr_floor = f32_from_orderable(o - (o == 0x80000000u ? 2u : 1u));
+    }
+  }
+  float thr_f = live ? thr_floor : INFINITY;
+  float best = -INFINITY;  // probe pass
+  int acc = 0;
+  uint32_t acc_phase = 0;
+  for (int t = rs; t < ntiles; t += p.n_rslots) {
+    const uint32_t row0 = p.row_begin + uint32_t(t) * K2_NT;
+    const int nvalid = int(min(uint32_t(K2_NT), p.row_end - row0));
+    mbar_wait(bar_tfull + acc * 8, acc_phase);
+    tc_fence_after();
+    if (warp_live) {
+#pragma unroll 1
+      for (int c = 0; c < K2_NT / 32; ++c) {
+        uint32_t v[32];
+        __syncwarp();
+        tmem_ld_x32(acc_tmem + (uint32_t(quarter * 32) << 16) + uint32_t(acc * K2_NT + c * 32), v);
+        tmem_wait_ld();
+        if constexpr (DUMP) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const int col = c * 32 + j;
+            if (col < nvalid && live)
+              p.dump[int64_t(qglob) * p.dump_ld + int64_t(row0 - p.row_begin) + col] = __uint_as_float(v[j]);
+          }
+        } else {
+          if (nvalid < K2_NT) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (c * 32 + j >= nvalid) v[j] = 0xFF800000u;  // -inf: rows past the segment end
+          }
+          // two-level filter: max per group of 8 columns, then max of the 4 groups against my k-th best
+          float gm[4];
+#pragma unroll
+          for (int g = 0; g < 4; ++g) {
+            float x = __uint_as_float(v[g * 8]);
+#pragma unroll
+            for (int j = 1; j < 8; ++j) x = fmaxf(x, __uint_as_float(v[g * 8 + j]));
+            gm[g] = x;
+          }
+          const float m = fmaxf(fmaxf(gm[0], gm[1]), fmaxf(gm[2], gm[3]));
+          if (p.probe_out != nullptr) {
+            best = fmaxf(best, m);
+          } else if (m > thr_f) {
+#pragma unroll
+            for (int g = 0; g < 4; ++g) {
+              if (gm[g] > thr_f) {
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                  const float s = __uint_as_float(v[g * 8 + j]);
+                  if (s > thr_f) {
+                    const uint64_t thr_key = k2_list_insert(mine, meta, k, make_key(s, row0 + uint32_t(c * 32 + g * 8 + j)));
+                    thr_f = thr_key ? fmaxf(thr_floor, key_score(thr_key)) : thr_floor;
+                  }
+                }
+              }
+            }
+          }
+        }
+      }
+    }
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) release(acc);
+    if (++acc == NACC) {
+      acc = 0;
+      acc_phase ^= 1u;
+    }
+  }
+  if constexpr (!DUMP) {
+    if (p.probe_out != nullptr) {
+      p.probe_out[size_t(qt * p.n_rslots + rs) * K2_BM + ql] = best;
+    } else {
+      uint64_t* dst = p.partial + (size_t(qt * p.n_rslots + rs) * K2_BM + ql) * k;
+      for (int j = 0; j < k; ++j) dst[j] = mine[size_t(j) * K2_BM];
+    }
+  }
 }
 
-// TS = true : the query tile is the A operand *in tensor memory* (128 lanes x D/2 packed-bf16 columns, written once
-//             by the epilogue threads with tcgen05.st); shared memory holds only the index ring (up to 13 x 16 KB
-//             in flight) and the tensor pipe reads half as many shared-memory bytes per MMA.  2 accumulators.
-// TS = false: the query tile is a shared-memory operand (TMA, SWIZZLE_128B), 4 accumulators.
-template <bool DUMP, bool TS>
+template <bool DUMP>
 __global__ void __launch_bounds__(K2_THREADS, 1)
 scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_x,
                  const UmmaParams p) {
@@ -213,16 +292,12 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
   // of the chain (prep / floor); only the warps that read what it wrote (queries, floors) or that write buffers it may
   // still read (partials, probe maxima) wait for it -- see the pdl_wait_prior_grid() calls below.
   pdl_launch_dependents();
-  constexpr int NACC = TS ? 2 : K2_ACC;
   const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
   const int ks = p.ks, nstages = p.nstages, k = p.k;
-  const int qslices = TS ? 0 : ks;                     // shared-memory slices taken by the query tile
-  const uint32_t acc_col0 = TS ? uint32_t(ks * 32) : 0u;  // TS: columns [0, D/2) hold the packed query tile
 
   const uint32_t q_s = smem_u32(smem);
-  const uint32_t st_s = q_s + uint32_t(qslices) * K2_SLICE;
-  uint64_t* lists = reinterpret_cast<uint64_t*>(smem + size_t(qslices + nstages) * K2_SLICE);  // [k][128]
+  const uint32_t st_s = q_s + uint32_t(ks) * K2_SLICE;
+  uint64_t* lists = reinterpret_cast<uint64_t*>(smem + size_t(ks + nstages) * K2_SLICE);  // [k][128]
   uint32_t* metas = reinterpret_cast<uint32_t*>(lists + size_t(k) * K2_BM);                     // [128]
   uint64_t* bars = reinterpret_cast<uint64_t*>(metas + K2_BM);
   const uint32_t bar_full = smem_u32(bars);                      // [K2_MAX_STAGES]
@@ -238,10 +313,6 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
   const int ntiles_all = int((nrows + K2_NT - 1) / K2_NT);
   // probe pass: only the first probe_tiles tiles of this CTA's strided sequence
   const int ntiles = p.probe_out ? min(ntiles_all, rs + p.probe_tiles * p.n_rslots) : ntiles_all;
-  // this CTA's tile sequence: [fused probe tiles (scanned for maxima only)] + [all of its tiles]
-  const int n_own = ntiles > rs ? (ntiles - rs + p.n_rslots - 1) / p.n_rslots : 0;
-  const int n_fprobe = min(p.fused_probe_tiles, n_own);
-  const int n_virt = n_own + n_fprobe;
 
   if (threadIdx.x == 0) {
     if ((q_s & 1023u) != 0) __trap();  // SWIZZLE_128B operands need 1024-byte alignment
@@ -253,9 +324,9 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
       mbar_init(bar_tfull + a * 8, 1);
       mbar_init(bar_tempty + a * 8, 4);  // one arrival per epilogue warp
     }
-    mbar_init(bar_q, TS ? 4 : 1);
+    mbar_init(bar_q, 1);
     fence_mbar_init();
-    if (!TS) tma_prefetch_desc(&tm_q);
+    tma_prefetch_desc(&tm_q);
     tma_prefetch_desc(&tm_x);
   }
   if (warp == 1) tmem_alloc_512(smem_u32(tmem_slot));
@@ -269,17 +340,14 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
     // The whole warp runs the (warp-uniform) loop; one elected lane issues the copies.  Keeping control flow
     // uniform lets the compiler hold addresses / coordinates in uniform registers.
     const bool leader = elect_one();
-    if constexpr (!TS) {
-      pdl_wait_prior_grid();   // the query tile was written by prep_queries_kernel
-      if (leader) {
-        mbar_arrive_expect_tx(bar_q, uint32_t(ks) * K2_SLICE);
-        for (int s = 0; s < ks; ++s) tma_load_2d(q_s + s * K2_SLICE, &tm_q, bar_q, s * 64, qt * K2_BM);
-      }
+    pdl_wait_prior_grid();   // the query tile was written by prep_queries_kernel
+    if (leader) {
+      mbar_arrive_expect_tx(bar_q, uint32_t(ks) * K2_SLICE);
+      for (int s = 0; s < ks; ++s) tma_load_2d(q_s + s * K2_SLICE, &tm_q, bar_q, s * 64, qt * K2_BM);
     }
     int stage = 0;
     uint32_t phase = 0;
-    for (int v = 0; v < n_virt; ++v) {
-      const int t = rs + (v < n_fprobe ? v : v - n_fprobe) * p.n_rslots;
+    for (int t = rs; t < ntiles; t += p.n_rslots) {
       const int32_t row0 = int32_t(p.row_begin + uint32_t(t) * K2_NT);
       for (int s = 0; s < ks; ++s) {
         mbar_wait(bar_empty + stage * 8, phase ^ 1u);
@@ -304,30 +372,20 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
     tc_fence_after();
     int stage = 0, acc = 0;
     uint32_t phase = 0, acc_phase = 0;
-    for (int v = 0; v < n_virt; ++v) {
+    for (int t = rs; t < ntiles; t += p.n_rslots) {
       mbar_wait(bar_tempty + acc * 8, acc_phase ^ 1u);
       tc_fence_after();
-      const uint32_t d_tmem = tmem_base + acc_col0 + uint32_t(acc) * K2_NT;
+      const uint32_t d_tmem = tmem_base + uint32_t(acc) * K2_NT;
       for (int s = 0; s < ks; ++s) {
         mbar_wait(bar_full + stage * 8, phase);
         tc_fence_after();
         const uint64_t b_desc = umma_smem_desc(st_s + stage * K2_SLICE);
-        if constexpr (TS) {
-          if (leader) {
+        const uint64_t a_desc = umma_smem_desc(q_s + s * K2_SLICE);
+        if (leader) {
 #pragma unroll
-            for (int kk = 0; kk < 4; ++kk)  // 16 bf16 of K = 8 packed TMEM columns of the query tile
-              umma_f16_ts(d_tmem, tmem_base + uint32_t(s * 32 + kk * 8), b_desc + uint64_t(kk * 2), idesc,
-                          uint32_t((s | kk) != 0));
-            umma_commit(bar_empty + stage * 8);
-          }
-        } else {
-          const uint64_t a_desc = umma_smem_desc(q_s + s * K2_SLICE);
-          if (leader) {
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk)  // 64-element slice = 4 x UMMA_K(16); +32 B per step inside the swizzle atom
-              umma_f16(d_tmem, a_desc + uint64_t(kk * 2), b_desc + uint64_t(kk * 2), idesc, uint32_t((s | kk) != 0));
-            umma_commit(bar_empty + stage * 8);
-          }
+          for (int kk = 0; kk < 4; ++kk)  // 64-element slice = 4 x UMMA_K(16); +32 B per step inside the swizzle atom
+            umma_f16(d_tmem, a_desc + uint64_t(kk * 2), b_desc + uint64_t(kk * 2), idesc, uint32_t((s | kk) != 0));
+          umma_commit(bar_empty + stage * 8);
         }
         __syncwarp();
         if (++stage == nstages) {
@@ -337,171 +395,16 @@ scan_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant
       }
       if (leader) umma_commit(bar_tfull + acc * 8);
       __syncwarp();
-      if (++acc == NACC) {
+      if (++acc == K2_ACC) {
         acc = 0;
         acc_phase ^= 1u;
       }
     }
   } else {
     // ------------------------------------------------------------------ epilogue: thread = query
-    const int quarter = warp & 3;              // TMEM lane quarter this warp may access
-    const int ql = quarter * 32 + lane;        // query within the tile
-    const int qglob = qt * K2_BM + ql;         // query within this launch
-    const bool live = qglob < p.B;
-    const bool warp_live = qt * K2_BM + quarter * 32 < p.B;   // any live query in this warp
-    pdl_wait_prior_grid();     // queries / floors come from the previous kernels; partials / probe maxima may still be read
-    if constexpr (TS) {
-      // stage the (already normalised, bf16) query tile into tensor memory: lane = query, column c = elements 2c, 2c+1
-      const uint32_t* qsrc = reinterpret_cast<const uint32_t*>(p.qbf16) + size_t(live ? qglob : 0) * (ks * 32);
-      for (int c = 0; c < ks; ++c) {
-        uint32_t w[32];
-#pragma unroll
-        for (int j = 0; j < 32; j += 4) {
-          uint4 x = live ? *reinterpret_cast<const uint4*>(qsrc + c * 32 + j) : make_uint4(0u, 0u, 0u, 0u);
-          w[j] = x.x; w[j + 1] = x.y; w[j + 2] = x.z; w[j + 3] = x.w;
-        }
-        tmem_st_x32(tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(c * 32), w);
-      }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_q);
-    }
-    uint64_t* mine = lists + ql;               // my candidate list: mine[j * 128], j = 0 .. k-1 (unsorted)
-    uint32_t* meta = metas + ql;
-    for (int j = 0; j < k; ++j) mine[size_t(j) * K2_BM] = 0ull;
-    *meta = 0u;
-    uint64_t thr_key = 0ull;
-    // Rows reach a thread in ascending order, so an equal score can never displace a held one: the strict
-    // compare `m > thr_f` is exact.  Padding queries never pass.
-    // A proven lower bound of the final k-th score (from the probe pass) pre-loads the filter, so the scan does
-    // not pay the warm-up in which every row beats an empty list.  `s >= floor` must pass: use the float just below.
-    float thr_floor = -INFINITY;
-    if (p.floor != nullptr && live) {
-      const float f = p.floor[qglob];
-      // the float just below f in the total order; below +-0 that is the largest negative subnormal, not -0.0
-      // (which compares equal to 0 and would reject every row scoring exactly 0, e.g. for an all-zero query)
-      if (f > -INFINITY) {
-        const uint32_t o = f32_orderable(f);
-        thr_floor = f32_from_orderable(o - (o == 0x80000000u ? 2u : 1u));
-      }
-    }
-    float thr_f = live ? thr_floor : INFINITY;
-    float best = -INFINITY;  // probe pass
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int vt = 0; vt < n_virt; ++vt) {
-      if (vt == n_fprobe && p.fused_probe_tiles > 0) {
-        // ---- end of the fused probe: publish this CTA's per-query maxima, meet every other CTA, derive the floor ----
-        // (a CTA with no tiles of its own still arrives; the producer / MMA warps do not wait here: they run ahead into
-        //  the real tiles until the accumulators are full)
-        p.probe_scratch[size_t(qt * p.n_rslots + rs) * K2_BM + ql] = best;
-        __threadfence();
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        if (ql == 0) {
-          atomicAdd(p.grid_barrier, 1u);
-          const uint64_t t0 = globaltimer_ns_k2();
-          while (*reinterpret_cast<volatile uint32_t*>(p.grid_barrier) < gridDim.x) {
-            if (globaltimer_ns_k2() - t0 > 20000000ull) break;   // 20 ms: never hang (two such grids on two streams could starve each
-                                                                // other of SMs); without the floor the scan is only slower
-            __nanosleep(64);
-          }
-          __threadfence();
-        }
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        const bool complete = *reinterpret_cast<volatile uint32_t*>(p.grid_barrier) >= gridDim.x;
-        if (live && complete && p.n_rslots >= k) {
-          // A cheap proven floor: split the CTA slots into k groups (slot mod k) and take each group's best score -- k scores
-          // of k DISTINCT rows -- so their minimum is a lower bound of the final k-th best score.  (Slightly weaker than the
-          // exact k-th largest the separate floor kernel computes, but it is 2 flops per value, branch-free, and every CTA
-          // has to derive it redundantly.)
-          float fl = INFINITY;
-          for (int g = 0; g < k; ++g) {
-            float mg = -INFINITY;
-            for (int r2 = g; r2 < p.n_rslots; r2 += k)
-              mg = fmaxf(mg, __ldcg(p.probe_scratch + size_t(qt * p.n_rslots + r2) * K2_BM + ql));
-            fl = fminf(fl, mg);
-          }
-          if (fl > -INFINITY && fl < INFINITY) {
-            const uint32_t o = f32_orderable(fl);
-            thr_floor = f32_from_orderable(o - (o == 0x80000000u ? 2u : 1u));
-            thr_f = thr_floor;
-          }
-        }
-        thr_key = 0ull;
-      }
-      const bool probing = p.probe_out != nullptr || vt < n_fprobe;
-      const int t = rs + (vt < n_fprobe ? vt : vt - n_fprobe) * p.n_rslots;
-      const uint32_t row0 = p.row_begin + uint32_t(t) * K2_NT;
-      const int nvalid = int(min(uint32_t(K2_NT), p.row_end - row0));
-      mbar_wait(bar_tfull + acc * 8, acc_phase);
-      tc_fence_after();
-      if (warp_live) {
-#pragma unroll 1
-        for (int c = 0; c < K2_NT / 32; ++c) {
-          uint32_t v[32];
-          __syncwarp();
-          tmem_ld_x32(tmem_base + (uint32_t(quarter * 32) << 16) + acc_col0 + uint32_t(acc * K2_NT + c * 32), v);
-          tmem_wait_ld();
-          if constexpr (DUMP) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-              const int col = c * 32 + j;
-              if (col < nvalid && live)
-                p.dump[int64_t(qglob) * p.dump_ld + int64_t(row0 - p.row_begin) + col] = __uint_as_float(v[j]);
-            }
-          } else {
-            if (nvalid < K2_NT) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j)
-                if (c * 32 + j >= nvalid) v[j] = 0xFF800000u;  // -inf: rows past the segment end
-            }
-            // two-level filter: max per group of 8 columns, then max of the 4 groups against my k-th best
-            float gm[4];
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              float x = __uint_as_float(v[g * 8]);
-#pragma unroll
-              for (int j = 1; j < 8; ++j) x = fmaxf(x, __uint_as_float(v[g * 8 + j]));
-              gm[g] = x;
-            }
-            const float m = fmaxf(fmaxf(gm[0], gm[1]), fmaxf(gm[2], gm[3]));
-            if (probing) {
-              best = fmaxf(best, m);
-            } else if (m > thr_f) {
-#pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                if (gm[g] > thr_f) {
-#pragma unroll
-                  for (int j = 0; j < 8; ++j) {
-                    const float s = __uint_as_float(v[g * 8 + j]);
-                    if (s > thr_f) {
-                      thr_key = k2_list_insert(mine, meta, k, make_key(s, row0 + uint32_t(c * 32 + g * 8 + j)));
-                      thr_f = thr_key ? fmaxf(thr_floor, key_score(thr_key)) : thr_floor;
-                    }
-                  }
-                }
-              }
-            }
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_tempty + acc * 8);
-      if (++acc == NACC) {
-        acc = 0;
-        acc_phase ^= 1u;
-      }
-    }
-    if constexpr (!DUMP) {
-      if (p.probe_out != nullptr) {
-        p.probe_out[size_t(qt * p.n_rslots + rs) * K2_BM + ql] = best;
-      } else {
-        uint64_t* dst = p.partial + (size_t(qt * p.n_rslots + rs) * K2_BM + ql) * k;
-        for (int j = 0; j < k; ++j) dst[j] = mine[size_t(j) * K2_BM];
-      }
-    }
+    pdl_wait_prior_grid();     // floors come from the previous kernels; partials / probe maxima may still be read
+    k2_epilogue<DUMP, K2_ACC>(p, qt, rs, ntiles, lists, metas, tmem_base, bar_tfull,
+                              [&](int acc) { mbar_arrive(bar_tempty + acc * 8); });
   }
   tc_fence_before();
   __syncthreads();
@@ -564,9 +467,8 @@ __global__ void probe_floor_kernel(const float* __restrict__ probe, int n_qtiles
 // fp32 queries -> L2-normalised bf16 (LanceDBStore._normalize, then narrowed for the tensor cores). Warp per query.
 template <typename E>
 __global__ void prep_queries_kernel(const float* __restrict__ q, E* __restrict__ out, int B, int dim,
-                                    float* __restrict__ qerr = nullptr, uint32_t* __restrict__ zero_word = nullptr) {
+                                    float* __restrict__ qerr = nullptr) {
   pdl_chain_prologue();
-  if (zero_word != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *zero_word = 0u;   // the scan's grid barrier
   const int lane = threadIdx.x & 31;
   const int qi = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (qi >= B) return;
@@ -646,13 +548,11 @@ inline size_t umma_align(size_t v) { return (v + 255) / 256 * 256; }
 
 inline int umma_qtiles(int B) { return (B + K2_BM - 1) / K2_BM; }
 
-constexpr size_t K2_PROGRESS_BYTES = 4096;  // lockstep counters: one u32 per CTA pair
-
 inline size_t umma_workspace_bytes(int sm_count, int dim, int B, int k) {
   const int qtiles = std::min(umma_qtiles(B), sm_count);
   const int ctas = std::max(sm_count, qtiles);
   return umma_align(size_t(B) * dim * 2) + umma_align(size_t(ctas) * K2_BM * k * 8) +
-         umma_align(size_t(ctas) * K2_BM * 4) + umma_align(size_t(B) * 4) + K2_PROGRESS_BYTES + 256;
+         umma_align(size_t(ctas) * K2_BM * 4) + umma_align(size_t(B) * 4) + 256;
 }
 
 inline int& umma_last_launches() {  // kernels launched by the last umma_search on this thread
@@ -662,8 +562,8 @@ inline int& umma_last_launches() {  // kernels launched by the last umma_search 
 inline int umma_launches_per_search() { return umma_last_launches(); }
 
 // smem plan: query tile + ring + lists + barriers
-inline int umma_plan_stages(int dim, int k, size_t* smem_bytes, bool ts = false) {
-  const int ks = ts ? 0 : dim / 64;
+inline int umma_plan_stages(int dim, int k, size_t* smem_bytes) {
+  const int ks = dim / 64;
   const size_t fixed = size_t(ks) * K2_SLICE + size_t(k) * K2_BM * 8 + K2_BM * 4 +
                        (2 * K2_MAX_STAGES + 2 * K2_ACC + 2) * 8 + 1024;
   int stages = int((size_t(K2_SMEM_LIMIT) - fixed) / K2_SLICE);
@@ -677,11 +577,7 @@ inline int umma_plan_stages(int dim, int k, size_t* smem_bytes, bool ts = false)
 // (same query precision, same per-row arithmetic) as the whole table and sharded results stay bit-identical.
 //   B <= 2  : K1 (fp32 queries, one launch, HBM-bound)      B >= 3, bf16/fp16 rows : K2 (16-bit queries on tcgen05)
 inline bool umma_preferred(int dtype, int dim, int B, int k, int64_t nrows) {
-  // MMR_FORCE_FAMILY=1|2 (measurement only, profiles/r01_k2_summary.md "crossover"): pin the family regardless of B
-  const int force = options().force_family;
-  const int min_b = force == 2 ? 1 : 3;
-  if (force == 1) return false;
-  if ((dtype != MMR_BF16 && dtype != MMR_F16) || dim % 64 != 0 || B < min_b) return false;
+  if ((dtype != MMR_BF16 && dtype != MMR_F16) || dim % 64 != 0 || B < 3) return false;
   if (nrows <= 0 || nrows >= (int64_t(1) << 31)) return false;
   return umma_plan_stages(dim, k, nullptr) >= 2;
 }

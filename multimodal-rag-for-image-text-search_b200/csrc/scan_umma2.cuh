@@ -8,7 +8,7 @@
 // Pair layout (cluster of 2 CTAs on one TPC):
 //   * CTA rank r owns query tile 2*pair + r: its 128 normalised bf16 queries live in ITS tensor memory (A operand,
 //     written with tcgen05.st), its accumulators D[128 x 128] live in ITS tensor memory, its epilogue warps filter
-//     ITS queries.  Lists / probe / floor logic is the same as K2's.
+//     ITS queries with K2's epilogue (k2_epilogue).
 //   * both CTAs stream the same row tiles; CTA r TMA-loads rows [row0 + 64 r, row0 + 64 r + 64) of each K-slice
 //     (8 KB, SWIZZLE_128B) into its own ring.  The loads use .cta_group::2 and signal the LEADER's "full" barrier.
 //   * only the leader (rank 0) issues tcgen05.mma.cta_group::2 (M=256, N=128, K=16); tcgen05.commit ... multicast
@@ -108,7 +108,6 @@ scan_umma2_kernel(const __grid_constant__ CUtensorMap tm_x, const UmmaParams p) 
   const uint32_t bar_tempty = bar_tfull + K2X_ACC * 8;            // [K2X_ACC]         used in the leader
   const uint32_t bar_q = bar_tempty + K2X_ACC * 8;                // [1]               used in the leader
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * K2X_MAX_STAGES + 2 * K2X_ACC + 1);
-  uint32_t* pace = tmem_slot + 2;   // [0] tiles started by this CTA's producer, [1] tiles it may start (lockstep window)
 
   const int pair = int(blockIdx.x >> 1);
   const int n_qpairs = (p.n_qtiles + 1) >> 1;
@@ -119,11 +118,7 @@ scan_umma2_kernel(const __grid_constant__ CUtensorMap tm_x, const UmmaParams p) 
   const int ntiles_all = int((nrows + K2_NT - 1) / K2_NT);
   const int ntiles = p.probe_out ? min(ntiles_all, rs + p.probe_tiles * p.n_rslots) : ntiles_all;
 
-  // lockstep (pair mode with several query pairs per row slot): gate = the non-lead CTA's producer, paced by its idle warp 1
-  const bool lockstep = p.progress != nullptr && p.probe_out == nullptr && !lead_cta && n_qpairs > 1;
   if (threadIdx.x == 0) {
-    pace[0] = 0u;
-    pace[1] = uint32_t(p.window);
     if ((st_s & 1023u) != 0) __trap();
     for (int s = 0; s < K2X_MAX_STAGES; ++s) {
       mbar_init(bar_full + s * 8, 1);
@@ -148,19 +143,7 @@ scan_umma2_kernel(const __grid_constant__ CUtensorMap tm_x, const UmmaParams p) 
     const bool leader = elect_one();
     int stage = 0;
     uint32_t phase = 0;
-    // lockstep with the other pairs of this row slot (they stream the same index tiles; see UmmaParams::progress): the
-    // NON-lead CTA's producer is the gate (the pair's MMAs need both halves of a tile), because that CTA's MMA warp is
-    // idle and can do the global polling -- this loop only reads shared memory.
-    uint32_t started = 0;
     for (int t = rs; t < ntiles; t += p.n_rslots) {
-      if (lockstep) {
-        if (leader) {
-          while (started >= *reinterpret_cast<volatile uint32_t*>(&pace[1])) __nanosleep(40);
-          *reinterpret_cast<volatile uint32_t*>(&pace[0]) = started + 1;
-        }
-        __syncwarp();
-      }
-      ++started;
       const int32_t row0 = int32_t(p.row_begin + uint32_t(t) * K2_NT + rank * K2X_HALF);
       for (int s = 0; s < ks; ++s) {
         mbar_wait(bar_empty + stage * 8, phase ^ 1u);
@@ -175,27 +158,8 @@ scan_umma2_kernel(const __grid_constant__ CUtensorMap tm_x, const UmmaParams p) 
         }
       }
     }
-    if (lockstep && leader) *reinterpret_cast<volatile uint32_t*>(&pace[0]) = 0xFFFFFFFFu;   // done
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer (leader CTA only)
-    if (!lead_cta && lockstep) {
-      // ---------------------------------------------------------------- pacer (this warp has no MMAs to issue)
-      // publishes this pair's progress, polls the other pairs of the row slot, and raises the producer's allowance
-      volatile uint32_t* prog = p.progress + size_t(rs) * n_qpairs;
-      if (lane == 0) {
-        for (;;) {
-          const uint32_t mine = *reinterpret_cast<volatile uint32_t*>(&pace[0]);
-          prog[qpair] = mine;
-          uint32_t slowest = 0xFFFFFFFFu;
-          for (int qp = 0; qp < n_qpairs; ++qp) slowest = min(slowest, prog[qp]);
-          *reinterpret_cast<volatile uint32_t*>(&pace[1]) =
-              slowest > 0xFFFFFFFFu - uint32_t(p.window) ? 0xFFFFFFFFu : slowest + uint32_t(p.window);
-          if (mine == 0xFFFFFFFFu) break;
-          __nanosleep(400);
-        }
-      }
-      __syncwarp();
-    }
     if (lead_cta) {
       const bool leader = elect_one();
       const uint32_t idesc = p.idesc;
@@ -235,117 +199,26 @@ scan_umma2_kernel(const __grid_constant__ CUtensorMap tm_x, const UmmaParams p) 
   } else {
     // ------------------------------------------------------------------ epilogue: thread = query (both CTAs)
     const int quarter = warp & 3;
-    const int ql = quarter * 32 + lane;
-    const int qglob = qt * K2_BM + ql;
+    const int qglob = qt * K2_BM + quarter * 32 + lane;
     const bool live = qglob < p.B;
-    const bool warp_live = qt * K2_BM + quarter * 32 < p.B;
-    const uint32_t lead_q = mapa_u32(bar_q, 0);
     pdl_wait_prior_grid();
-    {
-      const uint32_t* qsrc = reinterpret_cast<const uint32_t*>(p.qbf16) + size_t(live ? qglob : 0) * (ks * 32);
-      for (int c = 0; c < ks; ++c) {
-        uint32_t w[32];
+    // stage the (already normalised, bf16) query tile into tensor memory: lane = query, column c = elements 2c, 2c+1
+    const uint32_t* qsrc = reinterpret_cast<const uint32_t*>(p.qbf16) + size_t(live ? qglob : 0) * (ks * 32);
+    for (int c = 0; c < ks; ++c) {
+      uint32_t w[32];
 #pragma unroll
-        for (int j = 0; j < 32; j += 4) {
-          uint4 x = live ? *reinterpret_cast<const uint4*>(qsrc + c * 32 + j) : make_uint4(0u, 0u, 0u, 0u);
-          w[j] = x.x; w[j + 1] = x.y; w[j + 2] = x.z; w[j + 3] = x.w;
-        }
-        tmem_st_x32(tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(c * 32), w);
+      for (int j = 0; j < 32; j += 4) {
+        uint4 x = live ? *reinterpret_cast<const uint4*>(qsrc + c * 32 + j) : make_uint4(0u, 0u, 0u, 0u);
+        w[j] = x.x; w[j + 1] = x.y; w[j + 2] = x.z; w[j + 3] = x.w;
       }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(lead_q);
+      tmem_st_x32(tmem_base + (uint32_t(quarter * 32) << 16) + uint32_t(c * 32), w);
     }
-    uint64_t* mine = lists + ql;
-    uint32_t* meta = metas + ql;
-    for (int j = 0; j < k; ++j) mine[size_t(j) * K2_BM] = 0ull;
-    *meta = 0u;
-    uint64_t thr_key = 0ull;
-    float thr_floor = -INFINITY;
-    if (p.floor != nullptr && live) {
-      const float f = p.floor[qglob];
-      // the float just below f in the total order; below +-0 that is the largest negative subnormal, not -0.0
-      // (which compares equal to 0 and would reject every row scoring exactly 0, e.g. for an all-zero query)
-      if (f > -INFINITY) {
-        const uint32_t o = f32_orderable(f);
-        thr_floor = f32_from_orderable(o - (o == 0x80000000u ? 2u : 1u));
-      }
-    }
-    float thr_f = live ? thr_floor : INFINITY;
-    float best = -INFINITY;
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int t = rs; t < ntiles; t += p.n_rslots) {
-      const uint32_t row0 = p.row_begin + uint32_t(t) * K2_NT;
-      const int nvalid = int(min(uint32_t(K2_NT), p.row_end - row0));
-      mbar_wait(bar_tfull + acc * 8, acc_phase);
-      tc_fence_after();
-      if (warp_live && !p.skip_epi) {
-#pragma unroll 1
-        for (int c = 0; c < K2_NT / 32; ++c) {
-          uint32_t v[32];
-          __syncwarp();
-          tmem_ld_x32(tmem_base + (uint32_t(quarter * 32) << 16) + acc_col0 + uint32_t(acc * K2_NT + c * 32), v);
-          tmem_wait_ld();
-          if constexpr (DUMP) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-              const int col = c * 32 + j;
-              if (col < nvalid && live)
-                p.dump[int64_t(qglob) * p.dump_ld + int64_t(row0 - p.row_begin) + col] = __uint_as_float(v[j]);
-            }
-          } else {
-            if (nvalid < K2_NT) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j)
-                if (c * 32 + j >= nvalid) v[j] = 0xFF800000u;
-            }
-            float gm[4];
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              float x = __uint_as_float(v[g * 8]);
-#pragma unroll
-              for (int j = 1; j < 8; ++j) x = fmaxf(x, __uint_as_float(v[g * 8 + j]));
-              gm[g] = x;
-            }
-            const float m = fmaxf(fmaxf(gm[0], gm[1]), fmaxf(gm[2], gm[3]));
-            if (p.probe_out != nullptr) {
-              best = fmaxf(best, m);
-            } else if (m > thr_f) {
-#pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                if (gm[g] > thr_f) {
-#pragma unroll
-                  for (int j = 0; j < 8; ++j) {
-                    const float s = __uint_as_float(v[g * 8 + j]);
-                    if (s > thr_f) {
-                      thr_key = k2_list_insert(mine, meta, k, make_key(s, row0 + uint32_t(c * 32 + g * 8 + j)));
-                      thr_f = thr_key ? fmaxf(thr_floor, key_score(thr_key)) : thr_floor;
-                    }
-                  }
-                }
-              }
-            }
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(mapa_u32(bar_tempty + acc * 8, 0));
-      if (++acc == K2X_ACC) {
-        acc = 0;
-        acc_phase ^= 1u;
-      }
-    }
-    if constexpr (!DUMP) {
-      if (p.probe_out != nullptr) {
-        p.probe_out[size_t(qt * p.n_rslots + rs) * K2_BM + ql] = best;
-      } else {
-        uint64_t* dst = p.partial + (size_t(qt * p.n_rslots + rs) * K2_BM + ql) * k;
-        for (int j = 0; j < k; ++j) dst[j] = mine[size_t(j) * K2_BM];
-      }
-    }
+    tmem_wait_st();
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive_cluster(mapa_u32(bar_q, 0));
+    k2_epilogue<DUMP, K2X_ACC>(p, qt, rs, ntiles, lists, metas, tmem_base + acc_col0, bar_tfull,
+                               [&](int acc) { mbar_arrive_cluster(mapa_u32(bar_tempty + acc * 8, 0)); });
   }
   tc_fence_before();
   cluster_sync_all();  // the peer's shared memory / tensor memory stay alive until the leader's MMAs are done
@@ -374,10 +247,7 @@ inline int umma2_plan_stages(int k, size_t* smem_bytes) {
   return stages;
 }
 
-
 #ifdef __CUDACC__
-// One K2 search: prep queries -> scan (grid = qtiles x row slots) -> per-query merge.  `ws` is the K2 slice of the
-// workspace (umma_workspace_bytes).  dump != nullptr runs the raw-score debug variant instead of top-k.
 struct Umma2IndexState {
   bool valid = false;
   const void* rows = nullptr;
@@ -385,31 +255,22 @@ struct Umma2IndexState {
   CUtensorMap map;
 };
 
+// One K2 search: prep queries -> [probe pass -> floor] -> scan (grid = query tiles x row slots) -> per-query merge.  `ws` is
+// the K2 slice of the workspace (umma_workspace_bytes).  dump != nullptr runs the raw-score debug variant instead of top-k.
 inline int umma_search(UmmaIndexState& st, Umma2IndexState& st2, const void* rows, int64_t n_rows, int dim, int dtype, int sm_count,
                        const float* queries, int B, int k, uint32_t r0, uint32_t r1, int64_t row_base, float* out_s,
                        int64_t* out_r, uint8_t* ws, cudaStream_t stream, std::string& err, float* dump = nullptr,
                        int64_t dump_ld = 0, float* qerr = nullptr) {
-  if (!st.valid || st.rows != rows || st.n_rows != n_rows) {
-    if (!umma_make_map(&st.map, rows, n_rows, dim, dtype == MMR_BF16)) {
-      err = "cuTensorMapEncodeTiled failed for the index";
-      return MMR_ERR_CUDA;
-    }
-    st.valid = true;
-    st.rows = rows;
-    st.n_rows = n_rows;
-  }
-  // Operand placement, chosen from measurements on B200 (profiles/r01_k2_sweep.md): one query tile (B <= 128) is
-  // HBM-bound and fastest with both operands in shared memory and 4 accumulators; several query tiles are
-  // tensor-bound and fastest with the query tile in tensor memory (half the shared-memory reads per MMA, 13-deep
-  // ring).  MMR_UMMA_MODE=ss|ts overrides.
-  bool ts = umma_qtiles(B) > 1;
-  if (options().umma_mode == 1) ts = false;
-  if (options().umma_mode == 2) ts = true;
-  if (dim / 2 + 2 * K2_NT > 512) ts = false;
+  // Kernel, chosen from measurements on B200 (profiles/r01_k2_summary.md): one query tile (B <= 128) is HBM-bound and
+  // fastest on single CTAs with both operands in shared memory and 4 accumulators (scan_umma_kernel).  Several query tiles
+  // are tensor-bound: CTA pairs (cta_group::2) with the query tile in tensor memory (scan_umma2_kernel) read half the
+  // shared memory per MMA and are 5-9 % faster than single CTAs there (B=1024: 8.30 vs 8.72 ms).
+  const bool pair = umma_qtiles(B) >= 2;
   size_t smem_bytes = 0;
-  const int stages = umma_plan_stages(dim, k, &smem_bytes, ts);
-  if (stages < 2) {
-    err = "K2: shared memory plan does not fit";
+  const int stages = pair ? umma2_plan_stages(k, &smem_bytes) : umma_plan_stages(dim, k, &smem_bytes);
+  // the pair kernel's packed query tile (D/2 columns) and its accumulators share the 512 tensor-memory columns
+  if (stages < 2 || (pair && dim / 2 + K2X_ACC * K2_NT > 512)) {
+    err = "K2: shared / tensor memory plan does not fit";
     return MMR_ERR_UNSUPPORTED;
   }
   static bool attr_done[64] = {};
@@ -417,62 +278,67 @@ inline int umma_search(UmmaIndexState& st, Umma2IndexState& st2, const void* row
   cudaGetDevice(&cur_dev);
   bool& attr_set = attr_done[cur_dev & 63];
   if (!attr_set) {
-    cudaFuncSetAttribute(scan_umma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
-    cudaFuncSetAttribute(scan_umma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
-    cudaFuncSetAttribute(scan_umma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
-    cudaFuncSetAttribute(scan_umma_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
+    cudaFuncSetAttribute(scan_umma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
+    cudaFuncSetAttribute(scan_umma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
     cudaFuncSetAttribute(scan_umma2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
     cudaFuncSetAttribute(scan_umma2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2_SMEM_LIMIT);
     attr_set = true;
-  }
-  // CTA pairs (cta_group::2) for the tensor-bound regime (at least two query tiles): 5-9 % faster than cta_group::1
-  // there (B=1024: 8.30 vs 8.72 ms, profiles/r01_k2_summary.md).  MMR_UMMA_PAIR=0 falls back to single CTAs.
-  bool pair = ts && umma_qtiles(B) >= 2 && options().umma_pair != 0;
-  size_t smem2_bytes = 0;
-  const int stages2 = umma2_plan_stages(k, &smem2_bytes);
-  if (stages2 < 4) pair = false;
-  if (pair && (!st2.valid || st2.rows != rows || st2.n_rows != n_rows)) {
-    if (!umma2_make_map(&st2.map, rows, n_rows, dim, dtype == MMR_BF16)) {
-      err = "cuTensorMapEncodeTiled failed for the half-tile index map";
-      return MMR_ERR_CUDA;
-    }
-    st2.valid = true;
-    st2.rows = rows;
-    st2.n_rows = n_rows;
   }
   __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws);
   uint64_t* partial = reinterpret_cast<uint64_t*>(ws + umma_align(size_t(B) * dim * 2));
   const int ctas_max = std::max(sm_count, std::min(umma_qtiles(B), sm_count));
   float* probe = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(partial) + umma_align(size_t(ctas_max) * K2_BM * k * 8));
   float* floor = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(probe) + umma_align(size_t(ctas_max) * K2_BM * 4));
-  uint32_t* progress = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(floor) + umma_align(size_t(B) * 4));
-  const bool noprobe = options().umma_noprobe != 0;
-  uint32_t* grid_barrier = progress + K2_PROGRESS_BYTES / 4 - 16;   // last words of the counter block
-  if (dtype == MMR_BF16) launch_pdl(prep_queries_kernel<__nv_bfloat16>, dim3((B + 3) / 4), dim3(128), 0, stream, queries, qb, B, dim, qerr, grid_barrier);
-  else launch_pdl(prep_queries_kernel<__half>, dim3((B + 3) / 4), dim3(128), 0, stream, queries, reinterpret_cast<__half*>(qb), B, dim, qerr, grid_barrier);
+  if (pair) {
+    if (!st2.valid || st2.rows != rows || st2.n_rows != n_rows) {
+      if (!umma2_make_map(&st2.map, rows, n_rows, dim, dtype == MMR_BF16)) {
+        err = "cuTensorMapEncodeTiled failed for the half-tile index map";
+        return MMR_ERR_CUDA;
+      }
+      st2.valid = true;
+      st2.rows = rows;
+      st2.n_rows = n_rows;
+    }
+  } else {
+    if (!st.valid || st.rows != rows || st.n_rows != n_rows) {
+      if (!umma_make_map(&st.map, rows, n_rows, dim, dtype == MMR_BF16)) {
+        err = "cuTensorMapEncodeTiled failed for the index";
+        return MMR_ERR_CUDA;
+      }
+      st.valid = true;
+      st.rows = rows;
+      st.n_rows = n_rows;
+    }
+    // the query tile is TMA-loaded too (one tile, so one pass below)
+    if (!(st.q_valid && st.q_ptr == qb && st.q_rows == B)) {
+      if (!umma_make_map(&st.q_map, qb, B, dim, dtype == MMR_BF16)) {
+        err = "cuTensorMapEncodeTiled failed for the queries";
+        return MMR_ERR_CUDA;
+      }
+      st.q_valid = true;
+      st.q_ptr = qb;
+      st.q_rows = B;
+    }
+  }
+  // the scan kernel chosen above: top-k, or raw scores when prm.dump is set
+  auto launch_scan = [&](int grid, const UmmaParams& prm) {
+    const bool d = prm.dump != nullptr;
+    if (pair)
+      launch_pdl(d ? scan_umma2_kernel<true> : scan_umma2_kernel<false>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream,
+                 st2.map, prm);
+    else
+      launch_pdl(d ? scan_umma_kernel<true> : scan_umma_kernel<false>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream,
+                 st.q_map, st.map, prm);
+  };
+  if (dtype == MMR_BF16) launch_pdl(prep_queries_kernel<__nv_bfloat16>, dim3((B + 3) / 4), dim3(128), 0, stream, queries, qb, B, dim, qerr);
+  else launch_pdl(prep_queries_kernel<__half>, dim3((B + 3) / 4), dim3(128), 0, stream, queries, reinterpret_cast<__half*>(qb), B, dim, qerr);
   int launches = 1;
   const int max_q_per_pass = sm_count * K2_BM;
   for (int q0 = 0; q0 < B; q0 += max_q_per_pass) {
     const int bq = std::min(B - q0, max_q_per_pass);
-    CUtensorMap tm_q_local;
-    const void* qptr = qb + size_t(q0) * dim;
-    const bool cacheable = (q0 == 0);
-    if (!(cacheable && st.q_valid && st.q_ptr == qptr && st.q_rows == bq)) {
-      if (!umma_make_map(cacheable ? &st.q_map : &tm_q_local, qptr, bq, dim, dtype == MMR_BF16)) {
-        err = "cuTensorMapEncodeTiled failed for the queries";
-        return MMR_ERR_CUDA;
-      }
-      if (cacheable) {
-        st.q_valid = true;
-        st.q_ptr = qptr;
-        st.q_rows = bq;
-      }
-    }
-    const CUtensorMap& tm_q = cacheable ? st.q_map : tm_q_local;
     UmmaParams p{};
     p.ks = dim / 64;
-    p.idesc = umma_idesc_m128_n128(dtype == MMR_BF16);
-    p.nstages = options().umma_stages >= 2 ? std::min(stages, options().umma_stages) : stages;   // MMR_UMMA_STAGES: ring depth cap (measurement)
+    p.nstages = stages;
     p.k = k;
     p.B = bq;
     p.row_begin = r0;
@@ -482,57 +348,32 @@ inline int umma_search(UmmaIndexState& st, Umma2IndexState& st2, const void* row
     const int n_qpairs = (p.n_qtiles + 1) / 2;
     if (pair) {
       p.n_rslots = int(std::max<int64_t>(1, std::min<int64_t>((sm_count / 2) / n_qpairs, ntiles)));
-      p.nstages = stages2;
       p.idesc = umma_idesc_m256_n128(dtype == MMR_BF16);
     } else {
       p.n_rslots = int(std::max<int64_t>(1, std::min<int64_t>(sm_count / p.n_qtiles, ntiles)));
+      p.idesc = umma_idesc_m128_n128(dtype == MMR_BF16);
     }
     p.partial = partial;
     p.qbf16 = qb + size_t(q0) * dim;
     p.dump = dump ? dump + int64_t(q0) * dump_ld : nullptr;
     p.dump_ld = dump_ld;
-    p.skip_epi = options().umma_skip_epi;
     const int grid = pair ? 2 * n_qpairs * p.n_rslots : p.n_qtiles * p.n_rslots;
     // probe pass: worth it when every CTA streams many tiles (the warm-up it removes is ~k ln(n/k) inserts/thread)
     const int64_t tiles_per_cta = ntiles / p.n_rslots;
-    // Single-CTA kernel: the probe runs INSIDE the scan launch (first tiles scanned for maxima, grid barrier, floor) --
-    // two launches less on the latency-sensitive small-batch path.  MMR_UMMA_FUSED_PROBE=0 restores the separate pass.
-    const bool want_probe = !dump && !noprobe && tiles_per_cta >= 8 && p.n_rslots >= k;
-    const bool fused_probe = want_probe && !pair && options().umma_fused_probe && grid <= sm_count && q0 == 0 && bq == B;
-    if (fused_probe) {
-      p.fused_probe_tiles = int(std::max<int64_t>(1, std::min<int64_t>(16, tiles_per_cta / 24)));
-      p.probe_scratch = probe;
-      p.grid_barrier = grid_barrier;
-    }
-    if (want_probe && !fused_probe) {
+    if (!dump && tiles_per_cta >= 8 && p.n_rslots >= k) {
       launches += 2;
       UmmaParams pp = p;
       pp.probe_out = probe;
       pp.probe_tiles = int(std::max<int64_t>(1, std::min<int64_t>(16, tiles_per_cta / 24)));
-      if (pair) launch_pdl(scan_umma2_kernel<false>, dim3(grid), dim3(K2_THREADS), smem2_bytes, stream, st2.map, pp);
-      else if (ts) launch_pdl(scan_umma_kernel<false, true>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, pp);
-      else launch_pdl(scan_umma_kernel<false, false>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, pp);
+      launch_scan(grid, pp);
       const int wpb = 4;
       if (k <= 32) launch_pdl(probe_floor_kernel<1>, dim3((bq + wpb - 1) / wpb), dim3(wpb * 32), 0, stream, probe, p.n_qtiles, p.n_rslots, bq, k, floor + q0);
       else launch_pdl(probe_floor_kernel<2>, dim3((bq + wpb - 1) / wpb), dim3(wpb * 32), 0, stream, probe, p.n_qtiles, p.n_rslots, bq, k, floor + q0);
       p.floor = floor + q0;
     }
-    if (pair && n_qpairs > 1 && options().umma_lockstep && grid <= sm_count &&
-        size_t(p.n_rslots) * n_qpairs * 4 <= K2_PROGRESS_BYTES) {  // every CTA must be resident: waiting pairs spin
-      // (MMR_UMMA_LOCKSTEP=0 switches the lockstep window off: measurement)
-      cudaMemsetAsync(progress, 0, size_t(p.n_rslots) * n_qpairs * 4, stream);
-      p.progress = progress;
-      p.window = 24;   // tiles: 24 x 128 KB x row slots stays far inside the 126 MB L2
-    }
     launches += dump ? 1 : 2;
-    if (dump) {
-      if (pair) launch_pdl(scan_umma2_kernel<true>, dim3(grid), dim3(K2_THREADS), smem2_bytes, stream, st2.map, p);
-      else if (ts) launch_pdl(scan_umma_kernel<true, true>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, p);
-      else launch_pdl(scan_umma_kernel<true, false>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, p);
-    } else {
-      if (pair) launch_pdl(scan_umma2_kernel<false>, dim3(grid), dim3(K2_THREADS), smem2_bytes, stream, st2.map, p);
-      else if (ts) launch_pdl(scan_umma_kernel<false, true>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, p);
-      else launch_pdl(scan_umma_kernel<false, false>, dim3(grid), dim3(K2_THREADS), smem_bytes, stream, tm_q, st.map, p);
+    launch_scan(grid, p);
+    if (!dump) {
       const int wpb = 4;
       if (k <= 32)
         launch_pdl(merge_partials_kernel<1>, dim3((bq + wpb - 1) / wpb), dim3(wpb * 32), 0, stream, partial, p.n_qtiles,

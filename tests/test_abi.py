@@ -46,6 +46,9 @@ def test_argument_errors_have_messages():
     assert lib.mmr_merge_topk(None, None, 0, 1, 10, None, None, None) == 1
     assert lib.mmr_fuse(None, None, 0, None, None, 0, 0, 4, 0.25, None, None, None, None, None, None) == 1
     assert lib.mmr_search_workspace_bytes(None, 1, 10) == 0
+    assert lib.mmr_get_option(b"MMR_UMMA_LOCKSTEP") == -1                          # unknown switch
+    assert lib.mmr_set_option(b"MMR_UMMA_MODE", b"ts") == 1
+    assert b"unknown option" in lib.mmr_last_error()
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="CPU-only behaviour")

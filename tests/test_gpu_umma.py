@@ -23,23 +23,12 @@ def _bf16(x):
     return torch.from_numpy(x).to(torch.bfloat16).to(torch.float32).numpy()
 
 
-@pytest.fixture(params=["ts", "ss", "pair"])
-def umma_mode(request, monkeypatch):
-    """ts = query tile as the A operand in tensor memory; ss = both operands in shared memory;
-    pair = ts on CTA pairs (tcgen05.mma.cta_group::2, M = 256) for batches of at least two query tiles."""
-    import importlib
-    native = importlib.import_module("multimodal-rag-for-image-text-search_b200._native")
-    native.set_option("MMR_UMMA_MODE", "ts" if request.param == "pair" else request.param)
-    native.set_option("MMR_UMMA_PAIR", "1" if request.param == "pair" else "0")
-    yield request.param
-    native.set_option("MMR_UMMA_MODE", None)
-    native.set_option("MMR_UMMA_PAIR", None)
-
-
 @pytest.mark.parametrize("dim", [512, 384])
-def test_raw_scores_match_fp32_reference_of_same_inputs(mmr, dim, umma_mode):
+def test_raw_scores_match_fp32_reference_of_same_inputs(mmr, dim):
     """The tensor-core scores alone (no top-k): bf16 rows x bf16 unit queries, fp32 accumulate, against a plain
-    fp32 matmul of the same bf16 values.  Catches descriptor / swizzle / TMEM-layout mistakes directly."""
+    fp32 matmul of the same bf16 values.  Catches descriptor / swizzle / TMEM-layout mistakes directly.
+    b <= 128 runs the single-CTA kernel (both operands in shared memory), b = 131 the CTA-pair kernel (query tile in
+    tensor memory, tcgen05.mma.cta_group::2)."""
     n = 70_000 + 37           # last tile is partial
     rows = util.unit_rows(n, dim, seed=dim + 1)
     ix = mmr.ResidentIndex.from_f32(rows, dtype="bf16")
@@ -58,7 +47,7 @@ def test_raw_scores_match_fp32_reference_of_same_inputs(mmr, dim, umma_mode):
 
 
 @pytest.mark.parametrize("b", [5, 8, 127, 128, 129, 300])
-def test_topk_matches_oracle(mmr, b, umma_mode):
+def test_topk_matches_oracle(mmr, b):
     rows = util.unit_rows(150_000, 512, seed=91, cone=0.3)
     ix = mmr.ResidentIndex.from_f32(rows, dtype="bf16")
     qs = util.queries(b, 512, cone=0.3)
@@ -133,7 +122,7 @@ def test_k2_on_tiny_ranges(mmr, n):
 
 
 def test_k2_large_batch_parity(mmr):
-    """B = 1024 (8 query tiles, query tile in tensor memory, probe floor): a sample of queries against the oracle."""
+    """B = 1024 (8 query tiles on CTA pairs, query tile in tensor memory, probe floor): a sample of queries against the oracle."""
     rows = util.unit_rows(300_000, 512, seed=96, cone=0.3)
     ix = mmr.ResidentIndex.from_f32(rows, dtype="bf16")
     q = util.queries(1024, 512, cone=0.3)
