@@ -35,6 +35,12 @@ def main():
     parts_s = torch.stack([s, s]); parts_r = torch.stack([r, r + 100000])
     pkg.merge_topk(parts_s, parts_r)
     pkg.fuse((s, r), (s[:, :5].contiguous(), r[:, :5].contiguous()), 4, 0.25)
+    # image preprocessing: a ragged batch with a downscale, an upscale, one-pass and no-resize images and a partial tile
+    enc_mod = importlib.import_module("multimodal-rag-for-image-text-search_b200.encoders")
+    table = np.tile(np.arange(256, dtype=np.float32), (3, 1))
+    prep = enc_mod.DeviceImageProcessor(40, 40, 37, table)
+    rng = np.random.default_rng(0)
+    prep(images=[rng.integers(0, 256, (h, w, 3), dtype=np.uint8) for h, w in ((300, 170), (13, 29), (40, 41), (40, 40))])
     torch.cuda.synchronize()
     print("sanitize_small: done")
 

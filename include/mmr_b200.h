@@ -299,6 +299,30 @@ int mmr_encoder_create_vision(int device, const mmr_vision_config* config, mmr_e
 int mmr_encoder_forward_pixels(mmr_encoder* encoder, const float* pixels_dev, int32_t B, float* out_dev, void* stream);
 
 /*
+ * CLIP image preprocessing on the device, in front of mmr_encoder_forward_pixels: B decoded 8-bit RGB images of any sizes
+ * -> out_dev fp32 [B, 3, crop_h, crop_w] (NCHW), bit-identical to Pillow's Image.resize((out_w, out_h), BICUBIC) followed
+ * by a crop at (top, left) and the per-channel map table[c][byte] (HF CLIPImageProcessorPil: resize, centre crop, rescale,
+ * normalise; the caller computes the geometry and builds the table with HF's own rescale / normalise).
+ *   src_dev    the images, packed HWC RGB (3 bytes per pixel, rows contiguous), each starting at a multiple of 16 bytes
+ *              from a 16-byte aligned src_dev; the kernel reads whole 16-byte words, so each image's bytes rounded up to
+ *              a multiple of 16 must lie within src_bytes
+ *   geom_host  HOST array [B][7]: offset (bytes into src_dev), h, w, out_h, out_w (the resized size), top, left (the crop
+ *              window's origin in the resized image)
+ * Limits, checked with every other argument before any CUDA call (MMR_ERR_INVALID with a message): 1 <= crop_h, crop_w <=
+ * MMR_PREP_MAX_CROP; 1 <= h, w <= MMR_PREP_MAX_SIDE; 1 <= out_h, out_w <= MMR_PREP_MAX_OUT; top, left >= 0 with
+ * top + crop_h <= out_h and left + crop_w <= out_w; a downscale of at most 63.5x per axis (Pillow's bicubic window of
+ * 2 * ceil(2 * in / out) + 1 taps <= MMR_PREP_MAX_TAPS).  One launch per MMR_PREP_LAUNCH_IMAGES images, on `stream`.
+ */
+enum { MMR_PREP_MAX_CROP = 4096, MMR_PREP_MAX_SIDE = 65535, MMR_PREP_MAX_OUT = 1 << 24, MMR_PREP_MAX_TAPS = 255,
+       MMR_PREP_LAUNCH_IMAGES = 896 };
+typedef struct mmr_image_prep {
+  int32_t crop_h, crop_w;
+  float table[3][256];   /* pixel_values[c] = table[c][resized byte of channel c] */
+} mmr_image_prep;
+int mmr_image_preprocess(int device, const mmr_image_prep* cfg, const uint8_t* src_dev, int64_t src_bytes, const int64_t* geom_host,
+                         int32_t B, float* out_dev, void* stream);
+
+/*
  * Validation hook for the tensor-core path (K2): raw cosine scores of B queries against rows
  * [row_begin, row_end) as computed by the tcgen05 contraction (bf16 queries x bf16 rows, fp32 accumulate),
  * written to out_scores_dev[b * out_ld + (row - row_begin)].  workspace as for mmr_search(B, k = 10).

@@ -50,6 +50,7 @@ SYMBOLS = [
     ("mmr_encoder_forward", C.c_int, [_p, _p, _p, _p, _i32, _i32, _p, _p]),
     ("mmr_encoder_create_vision", C.c_int, [C.c_int, _p, C.POINTER(_p)]),
     ("mmr_encoder_forward_pixels", C.c_int, [_p, _p, _i32, _p, _p]),
+    ("mmr_image_preprocess", C.c_int, [C.c_int, _p, _p, _i64, _p, _i32, _p, _p]),
     ("mmr_fuse", C.c_int, [_p, _p, _i32, _p, _p, _i32, _i32, _i32, _f64, _p, _p, _p, _p, _p, _p]),
     ("mmr_fuse_f64", C.c_int, [_p, _p, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _f64, _p, _p, _p, _p]),
     ("mmr_debug_umma_scores", C.c_int, [_p, _p, _i32, _i64, _i64, _p, _i64, _p, _sz, _p]),
@@ -78,6 +79,11 @@ class VisionConfig(C.Structure):
     """mmr_vision_config (include/mmr_b200.h)."""
     _fields_ = [("hidden", _i32), ("layers", _i32), ("heads", _i32), ("intermediate", _i32), ("image_size", _i32),
                 ("patch_size", _i32), ("channels", _i32), ("proj_dim", _i32), ("ln_eps", C.c_float)]
+
+
+class ImagePrep(C.Structure):
+    """mmr_image_prep (include/mmr_b200.h)."""
+    _fields_ = [("crop_h", _i32), ("crop_w", _i32), ("table", (C.c_float * 256) * 3)]
 
 
 class NativeError(RuntimeError):

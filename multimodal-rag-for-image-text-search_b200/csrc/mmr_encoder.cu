@@ -9,6 +9,7 @@
 
 #include "abi_common.h"
 #include "encoder_kernels.cuh"
+#include "image_prep.cuh"
 
 using namespace mmr;
 #define fail mmr_fail
@@ -657,6 +658,71 @@ extern "C" int mmr_encoder_forward(mmr_encoder* e, const int32_t* input_ids_host
   CUDA_TRY(cudaMemcpyAsync(e->d_ids, e->h_stage, cap * 3 * 4, cudaMemcpyHostToDevice, st));
   if (e->cfg.hidden == 384) return forward_t<384>(e, B, S, out_dev, st);
   return forward_t<512>(e, B, S, out_dev, st);
+}
+
+// ------------------------------------------------------------------------------------------------ CLIP image preprocessing
+static_assert(sizeof(PrepParams) <= 32764, "the preprocessing geometry must fit the kernel parameters");
+static_assert(PREP_LAUNCH_IMAGES == MMR_PREP_LAUNCH_IMAGES && PREP_MAX_CHUNK * 2 <= PREP_RAW_BUDGET, "image_prep.cuh and the header");
+
+extern "C" int mmr_image_preprocess(int device, const mmr_image_prep* cfg, const uint8_t* src_dev, int64_t src_bytes,
+                                    const int64_t* geom_host, int32_t B, float* out_dev, void* stream) {
+  if (!cfg || !src_dev || !geom_host || !out_dev) return fail(MMR_ERR_INVALID, "NULL argument");
+  if (B < 1) return fail(MMR_ERR_INVALID, "B = %d: must be >= 1", B);
+  if (cfg->crop_h < 1 || cfg->crop_h > MMR_PREP_MAX_CROP || cfg->crop_w < 1 || cfg->crop_w > MMR_PREP_MAX_CROP)
+    return fail(MMR_ERR_INVALID, "crop %d x %d: each side must be in [1, %d]", cfg->crop_h, cfg->crop_w, int(MMR_PREP_MAX_CROP));
+  if ((reinterpret_cast<uintptr_t>(src_dev) & 15u) != 0) return fail(MMR_ERR_INVALID, "src_dev must be 16-byte aligned");
+  if ((reinterpret_cast<uintptr_t>(out_dev) & 3u) != 0) return fail(MMR_ERR_INVALID, "out_dev must be 4-byte aligned");
+  if (src_bytes < 16) return fail(MMR_ERR_INVALID, "src_bytes = %lld: too small for an image", (long long)src_bytes);
+  const int ch = cfg->crop_h, cw = cfg->crop_w;
+  for (int32_t i = 0; i < B; ++i) {
+    const int64_t* g = geom_host + 7 * int64_t(i);
+    const int64_t off = g[0], h = g[1], w = g[2], oh = g[3], ow = g[4], top = g[5], left = g[6];
+    if (h < 1 || h > MMR_PREP_MAX_SIDE || w < 1 || w > MMR_PREP_MAX_SIDE)
+      return fail(MMR_ERR_INVALID, "image %d: %lld x %lld pixels, each side must be in [1, %d]", i, (long long)h, (long long)w,
+                  int(MMR_PREP_MAX_SIDE));
+    if (oh < 1 || oh > MMR_PREP_MAX_OUT || ow < 1 || ow > MMR_PREP_MAX_OUT)
+      return fail(MMR_ERR_INVALID, "image %d: resized to %lld x %lld, each side must be in [1, %d]", i, (long long)oh, (long long)ow,
+                  int(MMR_PREP_MAX_OUT));
+    if (top < 0 || left < 0 || top + ch > oh || left + cw > ow)
+      return fail(MMR_ERR_INVALID, "image %d: crop %d x %d at (top %lld, left %lld) is not inside the resized %lld x %lld", i, ch, cw,
+                  (long long)top, (long long)left, (long long)oh, (long long)ow);
+    if (prep_taps(int(h), int(oh)) > MMR_PREP_MAX_TAPS || prep_taps(int(w), int(ow)) > MMR_PREP_MAX_TAPS)
+      return fail(MMR_ERR_INVALID, "image %d: %lld x %lld -> %lld x %lld downscales by more than 63.5x (bicubic window > %d taps)", i,
+                  (long long)h, (long long)w, (long long)oh, (long long)ow, int(MMR_PREP_MAX_TAPS));
+    if (off < 0 || off % 16 != 0 || off + ((h * w * 3 + 15) & ~int64_t(15)) > src_bytes)
+      return fail(MMR_ERR_INVALID, "image %d: offset %lld must be a multiple of 16 with its %lld bytes (rounded up to 16) inside src_bytes %lld",
+                  i, (long long)off, (long long)(h * w * 3), (long long)src_bytes);
+  }
+  CUDA_TRY(cudaSetDevice(device));
+  static bool attr_done[64] = {};
+  if (!attr_done[device & 63]) {
+    CUDA_TRY(cudaFuncSetAttribute(image_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    attr_done[device & 63] = true;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  static thread_local PrepParams p;   // 30 KB: off the stack
+  memcpy(p.table, cfg->table, sizeof(p.table));
+  p.crop_h = ch;
+  p.crop_w = cw;
+  for (int32_t b0 = 0; b0 < B; b0 += PREP_LAUNCH_IMAGES) {
+    const int n = std::min<int32_t>(PREP_LAUNCH_IMAGES, B - b0);
+    int span = 1;
+    p.taps_x = p.taps_y = 1;
+    for (int i = 0; i < n; ++i) {
+      const int64_t* g = geom_host + 7 * int64_t(b0 + i);
+      p.img[i] = PrepImage{g[0], int32_t(g[1]), int32_t(g[2]), int32_t(g[3]), int32_t(g[4]), int32_t(g[5]), int32_t(g[6])};
+      p.taps_x = std::max(p.taps_x, prep_taps(int(g[2]), int(g[4])));
+      p.taps_y = std::max(p.taps_y, prep_taps(int(g[1]), int(g[3])));
+      span = std::max(span, prep_span(int(g[2]), int(g[4]), PREP_COLS));
+    }
+    p.seg_bytes = (span * 3 + 15 + 15) & ~15;   // + up to 15 bytes in front of the segment's first pixel
+    p.chunk_rows = std::max(1, std::min(PREP_MAX_CHUNK, PREP_RAW_BUDGET / p.seg_bytes));
+    const dim3 grid((cw + PREP_COLS - 1) / PREP_COLS, (ch + PREP_ROWS - 1) / PREP_ROWS, n);
+    CUDA_TRY(launch_pdl(image_prep_kernel, grid, dim3(PREP_THREADS), prep_smem_bytes(p), st, p, src_dev,
+                        out_dev + size_t(b0) * 3 * ch * cw));
+    mmr_g_launches++;
+  }
+  return MMR_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ validation hooks

@@ -15,9 +15,10 @@ and the model of the ingest side, whose output fills the image rows the scan sea
     CLIP ViT-B/32 vision tower                                -> ImageEncoder       == embed_images_batch
 
 Weights come from the Hugging Face modules the reference loads (`from_hf_bert` / `from_hf_clip` /
-`from_hf_clip_vision` read their state_dict); tokenisation and image preprocessing stay on the host (any HF-style
-tokenizer, HF's CLIPImageProcessor).  There is no torch / CPU fallback: without the library or an sm_100 device
-construction raises.
+`from_hf_clip_vision` read their state_dict); tokenisation stays on the host (any HF-style tokenizer).  Image
+preprocessing runs either on the host (HF's CLIPImageProcessor) or on the device (DeviceImageProcessor, bit-identical to
+CLIPImageProcessorPil); decoding stays with the caller.  There is no torch / CPU fallback: without the library or an sm_100
+device construction raises.
 """
 from __future__ import annotations
 
@@ -306,8 +307,8 @@ class DeviceCrossEncoder:
 
 class ImageEncoder:
     """`embed_images_batch` (app/ml/embeddings.py:73-91) with the CLIP vision tower on the device: images -> unit-norm f32
-    [n, proj].  `processor` is the caller's HF CLIPImageProcessor (resize, centre crop, normalise stay on the host, as
-    tokenisation does for the text encoders); any callable returning {"pixel_values": [n, C, S, S]} works."""
+    [n, proj].  `processor` is the caller's HF CLIPImageProcessor (resize, centre crop, normalise on the host), a
+    DeviceImageProcessor (the same on the device), or any callable returning {"pixel_values": [n, C, S, S]}."""
 
     def __init__(self, processor: Callable, encoder: DeviceEncoder) -> None:
         self.processor, self.encoder = processor, encoder
@@ -324,5 +325,134 @@ class ImageEncoder:
         return np.concatenate(parts, axis=0)
 
 
-__all__ = ["DeviceEncoder", "TextQueryEncoder", "ImageQueryEncoder", "ImageEncoder", "DeviceCrossEncoder", "hf_bert_weights",
-           "hf_clip_text_weights", "hf_clip_vision_weights"]
+def clip_resize_geometry(h: int, w: int, shortest_edge: int, crop_h: int, crop_w: int) -> Tuple[int, int, int, int]:
+    """(out_h, out_w, top, left) of HF's CLIP preprocessing for an h x w image: the short side resized to shortest_edge, the
+    long side to int(shortest_edge * long / short) (transformers.image_transforms.get_resize_output_image_size), then the
+    centre crop's origin (image_transforms.center_crop)."""
+    short, long = (w, h) if w <= h else (h, w)
+    new_long = int(shortest_edge * long / short)
+    out_h, out_w = (new_long, shortest_edge) if w <= h else (shortest_edge, new_long)
+    return out_h, out_w, (out_h - crop_h) // 2, (out_w - crop_w) // 2
+
+
+def clip_value_table(do_rescale: bool, rescale_factor: float, do_normalize: bool, image_mean, image_std) -> np.ndarray:
+    """float32 [3, 256]: what the PIL backend's rescale and normalise make of each byte value of each channel, computed by
+    the same transformers functions on a [3, 1, 256] ramp (channels first, as the backend holds images)."""
+    from transformers.image_transforms import normalize, rescale
+    from transformers.image_utils import ChannelDimension
+    first = ChannelDimension.FIRST
+    x = np.broadcast_to(np.arange(256, dtype=np.uint8), (3, 1, 256)).copy()
+    if do_rescale:
+        x = rescale(x, rescale_factor, data_format=first, input_data_format=first)
+    if do_normalize:
+        x = normalize(x, image_mean, image_std, data_format=first, input_data_format=first)
+    return np.ascontiguousarray(x.reshape(3, 256), dtype=np.float32)
+
+
+def _field(d, key):
+    return d.get(key) if isinstance(d, dict) else getattr(d, key, None)
+
+
+class DeviceImageProcessor:
+    """CLIPImageProcessor on the device: decoded images (PIL images, or uint8 [H, W, 3] arrays) -> {"pixel_values": fp32
+    [n, 3, crop_h, crop_w] on the device}, bit-identical to CLIPImageProcessorPil (Pillow's bicubic resize of the short side,
+    centre crop, rescale, normalise).  A drop-in for the processor ImageEncoder takes.  Each call packs the images into one
+    reused pinned buffer, makes one host-to-device copy and one mmr_image_preprocess call on the current stream; decoding
+    stays with the caller."""
+
+    def __init__(self, shortest_edge: int, crop_h: int, crop_w: int, table: np.ndarray, device: Any = "cuda:0") -> None:
+        if not (0 < crop_h <= shortest_edge and 0 < crop_w <= shortest_edge):
+            raise ValueError(f"crop {crop_h} x {crop_w} must fit the resized short side {shortest_edge}")
+        table = np.asarray(table, dtype=np.float32)
+        if table.shape != (3, 256):
+            raise ValueError(f"table must be [3, 256], got {table.shape}")
+        N.lib()
+        if not torch.cuda.is_available():
+            raise N.NativeError("no CUDA device: the image preprocessing kernel has no CPU fallback")
+        self.shortest_edge, self.crop_h, self.crop_w = int(shortest_edge), int(crop_h), int(crop_w)
+        self.device = torch.device(device)
+        self.cfg = N.ImagePrep(self.crop_h, self.crop_w)
+        C.memmove(self.cfg.table, np.ascontiguousarray(table).ctypes.data, 3 * 256 * 4)
+        self._host: Optional[torch.Tensor] = None      # pinned staging, reused across calls
+        self._copied: Optional[torch.cuda.Event] = None
+
+    @staticmethod
+    def _hf_fields(processor) -> Tuple[int, int, int]:
+        """(shortest_edge, crop_h, crop_w) of a HF CLIP image processor (either backend), or ValueError naming the first
+        field whose effect the device path does not reproduce."""
+        from PIL import Image
+        if not getattr(processor, "do_resize", False):
+            raise ValueError("do_resize must be True: the device path always resizes")
+        size = getattr(processor, "size", None)
+        se = _field(size, "shortest_edge") if size is not None else None
+        if not se or any(_field(size, k) for k in ("height", "width", "longest_edge", "max_height", "max_width")):
+            raise ValueError(f"size must be {{'shortest_edge': n}} alone, got {size}")
+        if getattr(processor, "resample", None) != Image.Resampling.BICUBIC:
+            raise ValueError(f"resample {getattr(processor, 'resample', None)!r} is not supported (BICUBIC only)")
+        if not getattr(processor, "do_center_crop", False):
+            raise ValueError("do_center_crop must be True")
+        crop = getattr(processor, "crop_size", None)
+        ch, cw = (_field(crop, "height"), _field(crop, "width")) if crop is not None else (None, None)
+        if not ch or not cw:
+            raise ValueError(f"crop_size must give height and width, got {crop}")
+        if ch > se or cw > se:
+            raise ValueError(f"crop_size {ch} x {cw} is larger than size['shortest_edge'] {se}: the processor would pad")
+        if not getattr(processor, "do_convert_rgb", False):
+            raise ValueError("do_convert_rgb must be True: the device path takes RGB")
+        if getattr(processor, "do_pad", None):
+            raise ValueError("do_pad is not supported")
+        return int(se), int(ch), int(cw)
+
+    @classmethod
+    def from_hf(cls, processor, device: Any = "cuda:0") -> "DeviceImageProcessor":
+        """From a HF CLIPImageProcessor or CLIPImageProcessorPil; the output matches the PIL backend's bit for bit."""
+        se, ch, cw = cls._hf_fields(processor)
+        table = clip_value_table(bool(processor.do_rescale), processor.rescale_factor, bool(processor.do_normalize),
+                                 processor.image_mean, processor.image_std)
+        return cls(se, ch, cw, table, device=device)
+
+    @staticmethod
+    def _as_rgb_array(image) -> np.ndarray:
+        from PIL import Image
+        if isinstance(image, Image.Image):
+            return np.asarray(image if image.mode == "RGB" else image.convert("RGB"))
+        if isinstance(image, np.ndarray) and image.dtype == np.uint8 and image.ndim == 3 and image.shape[2] == 3:
+            return image
+        raise TypeError(f"expected a PIL image or a uint8 [H, W, 3] array, got {type(image).__name__}"
+                        + (f" {image.dtype} {image.shape}" if isinstance(image, np.ndarray) else ""))
+
+    def __call__(self, images=None, return_tensors: Optional[str] = "pt", **kwargs) -> Dict[str, torch.Tensor]:
+        if return_tensors != "pt":
+            raise ValueError(f"return_tensors must be 'pt' (device tensors), got {return_tensors!r}")
+        if kwargs:
+            raise TypeError(f"unsupported arguments: {sorted(kwargs)}")
+        arrays = [self._as_rgb_array(im) for im in (images if isinstance(images, (list, tuple)) else [images])]
+        if not arrays:
+            raise ValueError("no images")
+        geom = np.empty((len(arrays), 7), dtype=np.int64)
+        off = 0
+        for i, a in enumerate(arrays):
+            h, w = a.shape[:2]
+            geom[i] = (off, h, w, *clip_resize_geometry(h, w, self.shortest_edge, self.crop_h, self.crop_w))
+            off += (a.nbytes + 15) & ~15
+        with torch.cuda.device(self.device):
+            if self._copied is not None:
+                self._copied.synchronize()      # the previous call's upload may still read the staging buffer
+            if self._host is None or self._host.numel() < off:
+                self._host = torch.empty(max(off, 1 << 20), dtype=torch.uint8, pin_memory=True)
+            host = self._host.numpy()
+            for a, (o, h, w) in zip(arrays, geom[:, :3]):
+                np.copyto(host[o:o + h * w * 3].reshape(h, w, 3), a)
+            stream = torch.cuda.current_stream(self.device)
+            src = torch.empty(off, dtype=torch.uint8, device=self.device)
+            src.copy_(self._host[:off], non_blocking=True)
+            self._copied = torch.cuda.Event()
+            self._copied.record(stream)
+            out = torch.empty((len(arrays), 3, self.crop_h, self.crop_w), dtype=torch.float32, device=self.device)
+            N.check(N.lib().mmr_image_preprocess(self.device.index or 0, C.byref(self.cfg), src.data_ptr(), off, geom.ctypes.data,
+                                                 len(arrays), out.data_ptr(), stream.cuda_stream))
+        return {"pixel_values": out}
+
+
+__all__ = ["DeviceEncoder", "TextQueryEncoder", "ImageQueryEncoder", "ImageEncoder", "DeviceCrossEncoder", "DeviceImageProcessor",
+           "clip_resize_geometry", "clip_value_table", "hf_bert_weights", "hf_clip_text_weights", "hf_clip_vision_weights"]
